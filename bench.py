@@ -24,6 +24,10 @@ B200, so it is the workload at EVERY GPU count:
                 min-over-references, C5 dense full-length sweep: LOP3/POPC kernel vs tcgen05 int8 GEMM).
   --impl reference   the unmodified reference (oracle/_ref, built from /root/reference/src) timed on the host
                 cores on a bounded, DRAM-resident sample of the same workload (C1: the whole workload).
+  --steps K     the number of timed steps on every path. Lower it for --config C5 (each step runs both full-length sweeps,
+                ~11 s + ~4 s on one B200) and for --impl reference --config C1 (~2 min per step).
+  --dump-outputs DIR   the edge columns the last timed step returned, as DIR/<name>.npy: the inputs are seeded, so two builds
+                run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -168,10 +172,8 @@ def run_reference(args, saved_stdout):
     full = args.config == "C1"
     smp = RefSample(w, full=full)
     try:
-        if full:   # ~2 minutes per step: one timed step, whatever --steps says (stated in the line)
-            steps, warm = 1, 0
-        else:
-            steps, warm = args.steps, args.warmup
+        steps = args.steps
+        warm = 0 if full else args.warmup   # the whole C1 workload takes ~2 minutes per step: no warm-up steps
         smp.time_loader(mod, cores)
         for _ in range(warm):
             smp.step(mod, cores)
@@ -271,6 +273,31 @@ def _claim_stdout():
 def _emit(saved_fd, line):
     sys.stdout.flush()
     os.write(saved_fd, (json.dumps(line) + "\n").encode())
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, columns):
+    """--dump-outputs: writes the edge columns the timed path returned in its last step as <path>/<name>.npy, float64 (exact
+    for the integer columns), together with edge_index.npy, the position of each written edge in the full output. When all
+    of it would exceed DUMP_BYTES, every column keeps the same sample of edges, drawn with a fixed seed from the edge count,
+    so two builds run with the same arguments write files that can be compared one to one."""
+    cols = {k: np.asarray(v) for k, v in columns.items() if v is not None}
+    n = len(next(iter(cols.values())))
+    per_edge = 8 * (len(cols) + 1)
+    k = (DUMP_BYTES - 4096 * (len(cols) + 1)) // per_edge
+    idx = np.arange(n) if n <= k else np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+    os.makedirs(path, exist_ok=True)
+    for name, v in cols.items():
+        np.save(os.path.join(path, name + ".npy"), v[idx].astype(np.float64))
+    np.save(os.path.join(path, "edge_index.npy"), idx.astype(np.float64))
+
+
+def edge_columns(res):
+    """The per-edge numeric columns of an edge table (rows, cols, dist, filt, ncomp and, with dates, p0_log, eK, datediff).
+    The shared table of a multi-GPU run has no filt column: columns a table lacks are left out."""
+    return {k: res.get(k) for k in ("rows", "cols", "dist", "filt", "ncomp", "p0_log", "eK", "datediff")}
 
 
 def hbm_peak():
@@ -502,7 +529,14 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the forced full-length sweeps reported under roofline_kernels")
     ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--profile-phases", action="store_true", help="N>1: one extra untimed step with per-phase host timers (stages_ms.phases_ms)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the edge columns of the last timed step as DIR/<name>.npy (float64, at most 64 MB: a seeded sample of "
+                         "edges above that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the CUDA path computed (--impl b200)")
     if args.n or args.L:
         for c in CONFIGS.values():
             if args.n:
@@ -603,6 +637,8 @@ def main():
     clocks.mark()
     ms_per_step, wall_per_step, stats, res = timed(step, args.steps)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, edge_columns(res))
     value = replicas * P * L / (ms_per_step * 1e-3)
 
     def avg(k):

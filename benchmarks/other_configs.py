@@ -88,6 +88,8 @@ def run_c1(args, saved_stdout, B):
     clocks.mark()
     ms, res, stats = _timed(torch, step, args.steps, args.warmup)
     clk = clocks.stop()
+    if args.dump_outputs:
+        B.dump_outputs(args.dump_outputs, B.edge_columns(res))
     roof_pack, roof_sweep, pack_kernel = B.rooflines(tracs_b200, w, stats, peak, n, L, tc_peak, config=args.config if not (args.n or args.L) else None)
     line = _base_line(B, args, B.CONFIGS["C1"], "C1", P * L / (ms * 1e-3), ms, args.steps, args.warmup, clk,
                       int(sum(s["kernel_launches"] for s in stats)))
@@ -161,8 +163,8 @@ def run_c5(args, saved_stdout, B):
     clocks = B.Clocks(0)
     clocks.start()
     kernels, results, launches = {}, {}, 0
-    # the tensor-core kernel is the line's value: 3 warm-ups; the 11 s LOP3/POPC sweep is the comparison: one warm-up
-    plan = {"k_sweep_full_length": (1, 1), "k_sweep_tc_full_length": (max(1, min(args.steps, 3)), 3)}
+    # the faster kernel is the line's value; the tensor-core kernel gets 3 warm-ups, the 11 s LOP3/POPC sweep one
+    plan = {"k_sweep_full_length": (args.steps, 1), "k_sweep_tc_full_length": (args.steps, 3)}
     clocks.mark()
     for nm, variant in (("k_sweep_full_length", True), ("k_sweep_tc_full_length", "tc")):
         def step():
@@ -180,6 +182,8 @@ def run_c5(args, saved_stdout, B):
     best = min(results, key=lambda k: results[k][0])
     ms, res, stats = results[best]
     other = results[[k for k in results if k != best][0]][1]
+    if args.dump_outputs:
+        B.dump_outputs(args.dump_outputs, B.edge_columns(res))
     # the thresholded default path on the same input (prefilter + component blocks), for reference
     def dstep():
         return tracs_b200.pairsnp_packed(inp.buf.data_ptr(), n, L, inp.pitch, copy=False, **kw), tracs_b200.last_stats()
@@ -246,10 +250,12 @@ def run_c4(args, saved_stdout, B):
     clocks = B.Clocks(0)
     clocks.start()
     clocks.mark()
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     ms, out, stats = _timed(torch, step, steps, 2)
     clk = clocks.stop()
     oa, ob, ov, per = out
+    if args.dump_outputs:   # what the step hands back: the pairs after the min over references, in sample ids
+        B.dump_outputs(args.dump_outputs, {"rows": oa, "cols": ob, "dist": ov})
     line = _base_line(B, args, w, "C4", work / (ms * 1e-3), ms, steps, 2, clk, int(sum(s["kernel_launches"] for s in stats)))
     s = stats[-1]
     wp, t_sw = s["swept_wordpairs"], s["ms_sweep"]

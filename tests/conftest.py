@@ -40,11 +40,3 @@ def oracle_mod():
     from oracle import oracle
     oracle.lib()
     return oracle
-
-
-@pytest.fixture(scope="session")
-def ref_mod():
-    from oracle import refmod
-    if not refmod.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
-    return refmod.load()[0]

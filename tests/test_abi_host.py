@@ -146,11 +146,18 @@ def test_fasta_loader_record_semantics(oracle_mod, tmp_path):
         tracs_b200.read_fasta(str(tmp_path / "does_not_exist.fa"))
 
 
-def test_fasta_loader_live_reference_errors(ref_mod, tmp_path):
+def test_fasta_loader_live_reference_errors(oracle_mod, tmp_path):
+    """Ragged input: the reference's error, from the loader, the oracle and, where a local build of the reference exists
+    in oracle/_ref/ (not part of the repository), the unmodified reference module."""
+    from oracle import refmod
     p = str(tmp_path / "ragged.fa")
     open(p, "wb").write(b">a\nACGT\n>b\nACG\n")
-    with pytest.raises(RuntimeError, match="variable sequence lengths"):
-        ref_mod.pairsnp(fasta=[p], n_threads=1, dist=1, filter=False)
+    calls = [lambda: tracs_b200.read_fasta(p), lambda: oracle_mod.pairsnp([p], dist=1)]
+    if refmod.available():
+        calls.append(lambda: refmod.load()[0].pairsnp(fasta=[p], n_threads=1, dist=1, filter=False))
+    for call in calls:
+        with pytest.raises(RuntimeError, match="variable sequence lengths"):
+            call()
 
 
 def test_fasta_loader_large_roundtrip(tmp_path):

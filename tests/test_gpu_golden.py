@@ -82,6 +82,29 @@ def test_reference_kat_csv(tmp_path):
     assert rows[3][:4] == ["seq2", "seq3", "0.0", "1"] and rows[3][6:] == ["NA", "9", "kat"]
 
 
+def test_reference_test_assertions_on_reconstructed_fixture(tmp_path):
+    """The known answers of the reference's tests/test_llk.py, tests/test_pairsnp.py::test_pairsnp and
+    tests/test_trans_distance.py (the last two on their fixtures ambig.aln / dates_ambig.csv, reconstructed in
+    golden/ref_fixture/), through the drop-in module and the driver."""
+    from scipy.special import gammaln
+    from tracs_b200 import distance
+    fx = os.path.join(GOLD, "ref_fixture")
+    T = tracs_b200.install_dropin()
+    lp, lhs = T.lprob_k_given_N(N=7, k=4, delta=0.16963, lamb=3, beta=52, lgamma=gammaln(range(20)))
+    assert abs(lp + 17.9565184209608) < 1e-6 and abs(lhs - 12.0861694243766) < 1e-6
+    r = T.pairsnp(fasta=[os.path.join(fx, "ambig.aln")], n_threads=1, dist=10, filter=False)
+    assert all(isinstance(x, list) for x in r)
+    assert r[0] == [0, 0, 0, 0, 1, 1, 1, 2, 2, 3] and r[1] == [1, 2, 3, 4, 2, 3, 4, 3, 4, 4] and r[2] == [0, 2, 1, 1, 2, 2, 2, 3, 3, 0]
+    out = str(tmp_path / "ambig.csv")
+    distance.distance([os.path.join(fx, "ambig.aln")], out, metadata=os.path.join(fx, "dates_ambig.csv"), trans_threshold=10.0,
+                      snp_threshold=5)
+    l1, l2 = _rows(out)[1:3]
+    assert l1[:2] == ["seq1", "seq2"] and l2[:2] == ["seq1", "seq3"]
+    assert abs(float(l1[2]) - 0.002737907006988508) < 1e-6 and int(l1[3]) == 0 and int(l2[3]) == 2
+    assert abs(float(l1[4]) - 0.23794988406662973) < 1e-6 and abs(float(l2[4]) - 0.024467137572328577) < 1e-6
+    assert abs(float(l1[5]) - 2.6335200453700187) < 1e-6 and abs(float(l2[5]) - 7.315670110063259) < 1e-6
+
+
 def test_distance_cli_with_filter(tmp_path, ):
     # --filter: filtered column carries numbers, likelihood uses them; compare with the CPU oracle pipeline
     from oracle import oracle

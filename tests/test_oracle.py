@@ -104,7 +104,44 @@ def test_site_drop_rule_preserves_distances(oracle_mod):
     assert a[2].tolist() == b[2].tolist()
 
 
-def test_live_reference(oracle_mod, ref_mod, tmp_path):
+def _golden_alignment(name):
+    """Names and ASCII rows of a golden alignment (one header line per record, as synth.write_fasta writes it)."""
+    import gzip
+    names, rows = [], []
+    for ln in (gzip.open if name.endswith(".gz") else open)(os.path.join(GOLD, name), "rb"):
+        ln = ln.rstrip(b"\r\n")
+        if ln.startswith(b">"):
+            names.append(ln[1:].split()[0].decode())
+            rows.append([])
+        else:
+            rows[-1].append(ln)
+    return names, np.array([np.frombuffer(b"".join(r), np.uint8) for r in rows])
+
+
+def _local_reference():
+    """The unmodified reference module when a local build of it exists in oracle/_ref/ (not part of the repository), else None."""
+    from oracle import refmod
+    return refmod.load()[0] if refmod.available() else None
+
+
+def test_live_reference(oracle_mod, tmp_path):
+    """The oracle against the reference. Always: against the reference's outputs stored in golden.json (pairsnp at the
+    stored thresholds and with filter=True; the trans_dist grid, delta == 0 included, is compared in test_golden_trans_dist),
+    with every stored alignment re-written in each format the live comparison draws -- plain or gz, with or without header
+    descriptions, line width 0 / 60 / 7 -- and read with 1 to 3 threads. With a local build of the reference: also live, on
+    seeded random alignments."""
+    for filt, cases in ((False, G["pairsnp"]), (True, G["filter"])):
+        for case in cases:
+            names, s = _golden_alignment(case["fasta"])
+            exp = [case.get(k) for k in ("rows", "cols", "d", "names", "filt", "ncomp")]
+            for k in range(6):
+                p = str(tmp_path / ("k%d.fa%s" % (k, ".gz" if k % 2 else "")))
+                synth.write_fasta(p, s, names=names, width=[0, 60, 7][k % 3], descriptions=bool(k % 2))
+                r = oracle_mod.pairsnp([p], n_threads=1 + k % 3, dist=case["dist"], filter=filt)
+                assert all(e is None or r[t] == e for t, e in enumerate(exp)), (case["fasta"], k)
+    ref_mod = _local_reference()
+    if ref_mod is None:
+        return
     for trial in range(8):
         rng = np.random.default_rng(100 + trial)
         n, L = int(rng.integers(2, 30)), int(rng.integers(1, 700))
@@ -133,11 +170,17 @@ def test_live_reference(oracle_mod, ref_mod, tmp_path):
     assert np.allclose(b[1][~pos], (N[~pos] + 1) * 73.0 / 29.903, rtol=1e-9)
 
 
-def test_reconstructed_reference_fixture(ref_mod):
-    """tests/golden/ref_fixture/ambig.aln stands in for the absent fixture of the reference's tests/test_pairsnp.py:5-9:
-    on the UNMODIFIED reference module it gives exactly the vectors that test asserts."""
-    p = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_fixture", "ambig.aln")
-    r = ref_mod.pairsnp(fasta=[p], n_threads=1, dist=10, filter=False)
-    assert list(r[0]) == [0, 0, 0, 0, 1, 1, 1, 2, 2, 3]
-    assert list(r[1]) == [1, 2, 3, 4, 2, 3, 4, 3, 4, 4]
-    assert list(r[2]) == [0, 2, 1, 1, 2, 2, 2, 3, 3, 0]
+def test_reconstructed_reference_fixture(oracle_mod):
+    """tests/golden/ref_fixture/ambig.aln stands in for the absent fixture of the reference's tests/test_pairsnp.py:5-9: it
+    gives exactly the vectors that test asserts, on the oracle (held to the reference's stored outputs above) and, with a local
+    build of the reference, on the UNMODIFIED reference module itself."""
+    p = os.path.join(GOLD, "ref_fixture", "ambig.aln")
+    mods = [lambda: oracle_mod.pairsnp([p], n_threads=1, dist=10)]
+    ref_mod = _local_reference()
+    if ref_mod is not None:
+        mods.append(lambda: ref_mod.pairsnp(fasta=[p], n_threads=1, dist=10, filter=False))
+    for run in mods:
+        r = run()
+        assert list(r[0]) == [0, 0, 0, 0, 1, 1, 1, 2, 2, 3]
+        assert list(r[1]) == [1, 2, 3, 4, 2, 3, 4, 3, 4, 4]
+        assert list(r[2]) == [0, 2, 1, 1, 2, 2, 2, 3, 3, 0]
