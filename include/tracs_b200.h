@@ -129,6 +129,31 @@ int tracs_pairsnp_device(const uint8_t *dev_seqs, size_t n, size_t L, size_t pit
 int tracs_pairsnp_packed(const uint8_t *dev_nib, size_t n, size_t L, size_t pitch_bytes, const tracs_opts_t *opts,
                          tracs_edges_t *out);
 
+/* All-pairs SNP distance as a dense int32 matrix. d(i, j) is the `dist` column of tracs_pairsnp_* with
+ * dist = INT32_MAX: the number of sites where the two base masks share no base (src/pairsnp.hpp:393-403; N, gaps and
+ * unknown bytes match everything, IUPAC codes are honoured). Two shapes, chosen by opts->i_end / opts->j_start:
+ *   i_end = 0 or n, j_start = 0       -> n x n, symmetric, both triangles written, diagonal 0;
+ *   0 < i_end <= j_start < n          -> i_end x (n - j_start): rows = samples [0, i_end), cols = samples [j_start, n)
+ *                                        (the query x db mode of tracs_pairsnp with two files).
+ * out[r * ld + c]; entries of the padding (ld > cols) are never written. opts may be NULL (square matrix).
+ * opts->packed_input selects ASCII or 4-bit input as on the other entry points; opts->sweep_variant: 0 = tensor cores
+ * when the masks allow them, else LOP3/POPC; 1 = LOP3/POPC; 2 = tensor cores required (fails on 2-/3-base codes at
+ * variable sites). opts->want_ncomp is ignored. Errors, raised before any device call and naming the field: dist other
+ * than INT32_MAX, filter, want_trans / days, keep_on_device, shard_world > 1, any other (i_end, j_start), ld smaller
+ * than the column count, a bad pitch. A matrix that does not fit in device memory next to the ingest fails with a
+ * message that gives its size (no partial result). Not computed: the compared-sites count of every pair (use the
+ * thresholded pair list). */
+int tracs_distance_matrix_device(const uint8_t *dev_seqs, size_t n, size_t L, size_t pitch, const tracs_opts_t *opts,
+                                 int32_t *dev_out, size_t ld); /* device input (ASCII or packed), caller-owned device matrix */
+int tracs_distance_matrix_host(const uint8_t *seqs, size_t n, size_t L, size_t pitch, const tracs_opts_t *opts, int32_t *out,
+                               size_t ld); /* host input (streamed like tracs_pairsnp_host), host output */
+/* Host only: the matrix as text. First line: an empty cell, then the column names; then one line per row: the row
+ * name, then the values. sep = '\t' or ','. Names are written as given (no quoting, like tracs_write_distance_csv).
+ * Rows are formatted by parallel threads (TRACS_WRITE_THREADS, default: the hardware threads, at most 16); the bytes
+ * do not depend on their number. */
+int tracs_write_distance_matrix(const char *path, const int32_t *m, size_t rows, size_t cols, size_t ld,
+                                const char *const *row_names, const char *const *col_names, char sep);
+
 /* ASCII rows -> packed rows on the device (what the host-streaming path runs per chunk): dev_ascii[rows][pitch]
  * (pitch % 32 == 0, >= L rounded up to 32) -> dev_nib[rows][pitch_bytes]. Sites >= L become 1111. */
 int tracs_encode_packed(const uint8_t *dev_ascii, size_t rows, size_t L, size_t pitch, uint8_t *dev_nib, size_t pitch_bytes);

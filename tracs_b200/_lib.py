@@ -54,7 +54,8 @@ SYMBOLS = ["tracs_pairsnp", "tracs_pairsnp_host", "tracs_pairsnp_device", "tracs
            "tracs_memcpy_h2d", "tracs_int_peak", "tracs_read_fasta", "tracs_free_fasta", "tracs_shard_rowblocks",
            "tracs_site_shard_open", "tracs_site_shard_partials", "tracs_site_shard_close", "tracs_connected_components",
            "tracs_write_distance_csv", "tracs_float_repr", "tracs_pairsnp_packed", "tracs_encode_packed", "tracs_site_shard_finish", "tracs_tc_peak", "tracs_tc_peak_sustained", "tracs_site_shard_select", "tracs_site_shard_emit",
-           "tracs_host_register", "tracs_host_unregister"]
+           "tracs_host_register", "tracs_host_unregister", "tracs_distance_matrix_device", "tracs_distance_matrix_host",
+           "tracs_write_distance_matrix"]
 
 _lib = None
 
@@ -110,6 +111,10 @@ def lib():
         L.tracs_float_repr.argtypes = [C.c_double, C.c_char_p]
         L.tracs_float_repr.restype = C.c_size_t
         L.tracs_shard_rowblocks.argtypes = [C.c_uint32, C.c_int32, C.c_int32, C.c_void_p, C.POINTER(C.c_uint32)]
+        L.tracs_distance_matrix_device.argtypes = [C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.POINTER(Opts), C.c_void_p, C.c_size_t]
+        L.tracs_distance_matrix_host.argtypes = [C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.POINTER(Opts), C.c_void_p, C.c_size_t]
+        L.tracs_write_distance_matrix.argtypes = [C.c_char_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.POINTER(C.c_char_p),
+                                                  C.POINTER(C.c_char_p), C.c_char]
         _lib = L
     return _lib
 

@@ -151,6 +151,73 @@ def pairsnp_packed(dev_ptr, n, L, pitch_bytes, copy=True, **kw):
     return _lib.take_edges(e, names=False, copy=copy)
 
 
+def _dense_opts(n, n_query, packed, full_sweep):
+    """Options of the dense entry points: the square n x n matrix, or with n_query = q the q x (n - q) rectangle
+    (rows = samples [0, q), columns = samples [q, n)). Returns (opts, rows, cols)."""
+    if n_query is None:
+        return make_opts(packed=packed, full_sweep=full_sweep)[0], n, n
+    q = int(n_query)
+    if not 0 < q < n:
+        raise ValueError("n_query must satisfy 0 < n_query < n (rows = samples [0, n_query), columns = samples [n_query, n))")
+    return make_opts(i_end=q, j_start=q, packed=packed, full_sweep=full_sweep)[0], q, n - q
+
+
+def distance_matrix(seqs, n_query=None, packed=False, L=None, full_sweep=False):
+    """All-pairs SNP distances of a HOST alignment as a numpy int32 matrix: the `dist` column of pairsnp_* with
+    dist = INT32_MAX, for every pair. seqs: ASCII uint8[n][L], or with packed=True pack_nibbles rows (then L is
+    required). Square n x n (symmetric, zero diagonal), or with n_query = q the q x (n - q) query x db rectangle.
+    full_sweep: 0/False = tensor cores when the masks allow them, True = LOP3/POPC kernel, "tc" = tensor cores required."""
+    seqs = np.ascontiguousarray(seqs, dtype=np.uint8)
+    if seqs.ndim != 2:
+        raise ValueError("seqs must be a 2-D uint8 matrix")
+    n, width = seqs.shape
+    if packed and L is None:
+        raise ValueError("L (sites) is required with packed=True")
+    L = width if L is None else int(L)
+    o, rows, cols = _dense_opts(n, n_query, packed, full_sweep)
+    out = np.empty((rows, cols), np.int32)
+    _lib.check(_lib.lib().tracs_distance_matrix_host(seqs.ctypes.data, n, L, width, C.byref(o), out.ctypes.data, cols))
+    return out
+
+
+def distance_matrix_device(dev_ptr, n, L, pitch, out_ptr, ld, n_query=None, packed=False, full_sweep=False):
+    """All-pairs SNP distances of a DEVICE-resident alignment (ASCII, or 4-bit packed with packed=True) written into a
+    caller's device int32 buffer out_ptr (row r at out_ptr + 4 * r * ld), e.g. a torch int32 tensor's data_ptr().
+    Shapes as distance_matrix; padding columns (ld > cols) are not written."""
+    o, _, _ = _dense_opts(int(n), n_query, packed, full_sweep)
+    _lib.check(_lib.lib().tracs_distance_matrix_device(C.c_void_p(dev_ptr), int(n), int(L), int(pitch), C.byref(o), C.c_void_p(out_ptr),
+                                                       int(ld)))
+
+
+def write_distance_matrix(path, m, row_names, col_names, sep="\t", n_threads=None):
+    """Writes an int32 matrix as text through the native writer: a header line (an empty cell, then the column names),
+    then one line per row (its name, then the values). sep is "\\t" or ","; names are written as given. A row-strided
+    view (m = big[:, :cols]) is written without a copy. n_threads: formatting threads (the output does not depend on it)."""
+    m = np.asarray(m)
+    if m.ndim != 2:
+        raise ValueError("m must be a 2-D matrix")
+    if m.dtype != np.int32 or m.strides[1] != 4 or m.strides[0] % 4 or m.strides[0] < 4 * m.shape[1]:
+        m = np.ascontiguousarray(m, dtype=np.int32)
+    rows, cols = m.shape
+    ld = max(cols, m.strides[0] // 4) if rows > 1 else cols
+    if len(row_names) != rows or len(col_names) != cols:
+        raise ValueError("need one name per row (%d) and per column (%d)" % (rows, cols))
+    rn = (C.c_char_p * max(1, rows))(*[str(s).encode() for s in row_names])
+    cn = (C.c_char_p * max(1, cols))(*[str(s).encode() for s in col_names])
+    old = os.environ.get("TRACS_WRITE_THREADS")
+    if n_threads is not None:
+        os.environ["TRACS_WRITE_THREADS"] = str(int(n_threads))
+    try:
+        _lib.check(_lib.lib().tracs_write_distance_matrix(os.fsencode(os.fspath(path)), m.ctypes.data, rows, cols, ld, rn, cn,
+                                                          sep.encode()))
+    finally:
+        if n_threads is not None:
+            if old is None:
+                os.environ.pop("TRACS_WRITE_THREADS", None)
+            else:
+                os.environ["TRACS_WRITE_THREADS"] = old
+
+
 def min_over_refs(a, b, val):
     """Min-over-references combine (SURVEY A.6): unordered (a,b) -> min(val). Sorted by (lo, hi)."""
     a = np.ascontiguousarray(a, dtype=np.uint64)

@@ -700,6 +700,189 @@ int tracs_pairsnp_host(const uint8_t *seqs, size_t n, size_t L, size_t pitch, co
   });
 }
 
+}  // extern "C"
+
+// ---- dense distance matrix (tracs_distance_matrix_*) ----------------------------------------------------
+namespace tracs {
+struct DenseShape {
+  uint64_t rows = 0, cols = 0;
+};
+// Argument check of the dense entry points. Host code only (no device call), so it runs before require_device().
+static DenseShape dense_check(const tracs_opts_t *opts, size_t n, size_t L, size_t pitch, size_t ld, const void *out, bool host_input) {
+  const tracs_opts_t o = normalise(opts, n);
+  const char *pre = "distance matrix: ";
+  if (o.dist != INT32_MAX)
+    throw std::runtime_error(std::string(pre) + "opts->dist must be INT32_MAX (every pair); a threshold is what tracs_pairsnp_* is for");
+  if (o.filter) throw std::runtime_error(std::string(pre) + "opts->filter (recombination filter) applies to the thresholded pair list only");
+  if (o.want_trans || o.days) throw std::runtime_error(std::string(pre) + "opts->want_trans / opts->days (transmission likelihood) apply to the thresholded pair list only");
+  if (o.keep_on_device) throw std::runtime_error(std::string(pre) + "opts->keep_on_device applies to the edge list only");
+  if (o.shard_world > 1) throw std::runtime_error(std::string(pre) + "opts->shard_world > 1: the dense matrix is computed on one GPU");
+  if (o.sweep_variant < 0 || o.sweep_variant > 2) throw std::runtime_error(std::string(pre) + "opts->sweep_variant must be 0, 1 or 2");
+  if (n >= (1ull << 31)) throw std::runtime_error(std::string(pre) + "n: too many samples");
+  const uint64_t i_end = opts ? opts->i_end : 0, j_start = opts ? opts->j_start : 0;
+  DenseShape sh;
+  if ((i_end == 0 || i_end == n) && j_start == 0) {
+    sh.rows = sh.cols = n;  // square
+  } else if (i_end >= 1 && j_start >= i_end && j_start < n) {
+    sh.rows = i_end;  // query x db rectangle
+    sh.cols = n - j_start;
+  } else {
+    throw std::runtime_error(std::string(pre) + "opts->i_end / opts->j_start: either i_end = 0 or n with j_start = 0 (square matrix), or "
+                             "0 < i_end <= j_start < n (rows [0, i_end) x cols [j_start, n))");
+  }
+  if (ld < sh.cols) throw std::runtime_error(std::string(pre) + "ld (" + std::to_string(ld) + ") is smaller than the column count (" + std::to_string(sh.cols) + ")");
+  if (!out && sh.rows && sh.cols) throw std::runtime_error(std::string(pre) + "out is NULL");
+  const bool packed = o.packed_input != 0;
+  bool pitch_ok;
+  if (host_input) pitch_ok = packed ? pitch >= (L + 1) / 2 : pitch >= L;
+  else if (packed) pitch_ok = pitch % 16 == 0 && pitch * 2 >= std::max<size_t>(32, (L + 31) / 32 * 32);
+  else pitch_ok = pitch % 32 == 0 && pitch >= (L + 31) / 32 * 32;
+  if (!pitch_ok && n > 0)
+    throw std::runtime_error(std::string(pre) + "pitch (" + std::to_string(pitch) + ") " +
+                             (host_input ? (packed ? "must hold (L + 1) / 2 bytes" : "must be >= L")
+                                         : (packed ? "must be a multiple of 16 bytes and hold L rounded up to 32 sites"
+                                                   : "must be a multiple of 32 and >= L rounded up to 32")));
+  return sh;
+}
+
+static std::string dense_too_large(uint64_t rows, uint64_t cols) {
+  size_t free_b = 0, total_b = 0;
+  if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) cudaGetLastError();
+  char b[512];
+  snprintf(b, sizeof b,
+           "distance matrix: a %llu x %llu int32 matrix (%.1f GB) and the ingest of the alignment do not fit in device memory "
+           "(%.1f GB on the device): for an alignment this large ask for the thresholded pair list (tracs_pairsnp_* with a finite dist)",
+           (unsigned long long)rows, (unsigned long long)cols, (double)rows * (double)cols * 4.0 / 1e9, (double)total_b / 1e9);
+  return b;
+}
+
+// a device allocation that fails inside the call becomes the "does not fit" message (the buffers already taken go back
+// to the cache on the way out, so the library stays usable)
+template <typename F>
+static void dense_fit_guard(uint64_t rows, uint64_t cols, F &&f) {
+  try {
+    f();
+  } catch (const CudaError &e) {
+    if (e.msg.find("cudaErrorMemoryAllocation") == std::string::npos) throw;
+    cudaGetLastError();
+    throw std::runtime_error(dense_too_large(rows, cols));
+  }
+}
+}  // namespace tracs
+
+extern "C" {
+
+int tracs_distance_matrix_device(const uint8_t *dev_seqs, size_t n, size_t L, size_t pitch, const tracs_opts_t *opts, int32_t *dev_out,
+                                 size_t ld) {
+  memset(&g_stats, 0, sizeof g_stats);
+  return guarded([&] {
+    const DenseShape sh = dense_check(opts, n, L, pitch, ld, dev_out, false);
+    require_device();
+    InterruptScope sigint;
+    if (sh.rows == 0 || sh.cols == 0) return;
+    const tracs_opts_t o = normalise(opts, n);
+    dense_fit_guard(sh.rows, sh.cols, [&] { distance_matrix_device(dev_seqs, n, L, pitch, o, dev_out, ld, 0); });
+  });
+}
+
+int tracs_distance_matrix_host(const uint8_t *seqs, size_t n, size_t L, size_t pitch, const tracs_opts_t *opts, int32_t *out,
+                               size_t ld) {
+  memset(&g_stats, 0, sizeof g_stats);
+  return guarded([&] {
+    const DenseShape sh = dense_check(opts, n, L, pitch, ld, out, true);
+    require_device();
+    InterruptScope sigint;
+    if (sh.rows == 0 || sh.cols == 0) return;
+    tracs_opts_t o = normalise(opts, n);
+    const uint64_t m_bytes = sh.rows * sh.cols * 4, in_bytes = (uint64_t)n * std::max<uint64_t>(16, (L + 31) / 32 * 16);
+    size_t free_b = 0, total_b = 0;
+    TRACS_CK(cudaMemGetInfo(&free_b, &total_b));
+    if (m_bytes + in_bytes > total_b) throw std::runtime_error(dense_too_large(sh.rows, sh.cols));
+    dense_fit_guard(sh.rows, sh.cols, [&] {
+      DevBuf<int32_t> m(sh.rows * sh.cols);  // library-owned, ld = cols
+      {
+        DevBuf<uint8_t> nib;
+        size_t pitch4 = 0;
+        stream_host_to_packed(seqs, n, L, pitch, o.packed_input != 0, nib, pitch4, 0);
+        o.packed_input = 1;
+        distance_matrix_device(nib.p, n, L, pitch4, o, m.p, sh.cols, 0);
+      }
+      Timer T(0);
+      T.start();
+      TRACS_CK(cudaMemcpy2DAsync(out, ld * 4, m.p, sh.cols * 4, sh.cols * 4, sh.rows, cudaMemcpyDeviceToHost, 0));
+      TRACS_CK(cudaStreamSynchronize(0));
+      g_stats.ms_d2h += T.stop();
+      g_stats.ms_total += g_stats.ms_d2h;
+      g_stats.d2h_bytes += m_bytes;
+    });
+  });
+}
+
+int tracs_write_distance_matrix(const char *path, const int32_t *m, size_t rows, size_t cols, size_t ld, const char *const *row_names,
+                                const char *const *col_names, char sep) {
+  return guarded([&] {
+    if (sep != '\t' && sep != ',') throw std::runtime_error("write_distance_matrix: sep must be '\\t' or ','");
+    if (ld < cols) throw std::runtime_error("write_distance_matrix: ld is smaller than the column count");
+    if (!m && rows && cols) throw std::runtime_error("write_distance_matrix: m is NULL");
+    if ((rows && !row_names) || (cols && !col_names)) throw std::runtime_error("write_distance_matrix: names are NULL");
+    for (size_t r = 0; r < rows; ++r)
+      if (!row_names[r]) throw std::runtime_error("write_distance_matrix: a row name is NULL");
+    for (size_t c = 0; c < cols; ++c)
+      if (!col_names[c]) throw std::runtime_error("write_distance_matrix: a column name is NULL");
+    std::unique_ptr<FILE, int (*)(FILE *)> f(fopen(path, "wb"), fclose);
+    if (!f) throw std::runtime_error(std::string("cannot open ") + path);
+    std::string head;
+    for (size_t c = 0; c < cols; ++c) {
+      head += sep;
+      head += col_names[c];
+    }
+    head += '\n';
+    if (fwrite(head.data(), 1, head.size(), f.get()) != head.size()) throw std::runtime_error("write error");
+    // rows are formatted by T threads, a batch of T consecutive row ranges at a time, and written in row order: the bytes
+    // do not depend on T (TRACS_WRITE_THREADS, default: the hardware threads, at most 16)
+    const char *env_t = getenv("TRACS_WRITE_THREADS");
+    const unsigned hw = std::max(1u, std::thread::hardware_concurrency());
+    const size_t T = env_t ? (size_t)std::max(1, atoi(env_t)) : (size_t)std::min(16u, hw);
+    const size_t rows_per = std::max<size_t>(1, ((size_t)4 << 20) / (cols * 12 + 64));  // ~4 MB of text per range
+    std::vector<std::string> bufs(T);
+    for (size_t r0 = 0; r0 < rows; r0 += T * rows_per) {
+      auto format = [&](size_t t) {
+        std::string &b = bufs[t];
+        b.clear();
+        const size_t a = r0 + t * rows_per, e = std::min(rows, a + rows_per);
+        char num[16];
+        for (size_t r = a; r < e; ++r) {
+          b += row_names[r];
+          const int32_t *row = m + r * ld;
+          for (size_t c = 0; c < cols; ++c) {
+            b += sep;
+            b.append(num, (size_t)(std::to_chars(num, num + sizeof num, row[c]).ptr - num));
+          }
+          b += '\n';
+        }
+      };
+      const size_t used = std::min(T, (rows - r0 + rows_per - 1) / rows_per);
+      std::vector<char> failed(used, 0);
+      std::vector<std::thread> pool;
+      for (size_t t = 1; t < used; ++t)
+        pool.emplace_back([&, t] {
+          try {
+            format(t);
+          } catch (...) {
+            failed[t] = 1;
+          }
+        });
+      format(0);
+      for (auto &th : pool) th.join();
+      for (char x : failed)
+        if (x) throw std::bad_alloc();
+      for (size_t t = 0; t < used; ++t)
+        if (fwrite(bufs[t].data(), 1, bufs[t].size(), f.get()) != bufs[t].size()) throw std::runtime_error("write error");
+    }
+    if (fclose(f.release()) != 0) throw std::runtime_error("write error");
+  });
+}
+
 int tracs_pairsnp(const char *const *paths, int n_paths, int n_threads, int32_t dist, int filter,
                   tracs_edges_t *out) {
   memset(out, 0, sizeof *out);

@@ -307,6 +307,9 @@ struct HostEdges {
 std::shared_ptr<const std::vector<double>> lgamma_table(size_t n);  // lg[x] = lgamma(x), x < n; immutable snapshot
 void sweep_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint64_t pitch, const tracs_opts_t &o,
                   HostEdges &out, cudaStream_t st);
+// every pair's distance into a dense int32 device matrix (tracs_distance_matrix_device; arguments validated by the caller)
+void distance_matrix_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint64_t pitch, const tracs_opts_t &o, int32_t *out,
+                            uint64_t ld, cudaStream_t st);
 
 // last step of the site-sharded sweep (shard.inl): summed candidate vectors -> edge columns
 void site_shard_finish_device(const uint64_t *dev_keys, const uint32_t *dev_d, const uint32_t *dev_union, uint64_t n_keys, uint64_t n,

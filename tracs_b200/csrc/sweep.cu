@@ -5,6 +5,7 @@
 //   K0b k_gather    variable sites only -> interleaved A/C/G/T bit-planes P[word][sample] (uint4)
 //   K1  k_sweep     128x128 pair tiles, bulk-async (TMA engine, UBLKCP) staged panels, 8x8 register
 //                   micro-tiles, LOP3 + POPC, fused threshold + edge append  [INT-pipe bound]
+//                   (k_sweep<true>: every distance stored into a dense matrix instead, distance_matrix_device)
 //   K2  k_ncomp     compared-site count for emitted edges via block-sparse N-plane intersection
 //
 // Semantics restated from the reference (paths relative to gtonkinhill/tracs):
@@ -618,10 +619,25 @@ struct SweepArgs {
   uint32_t cb_min;  // first col-block allowed by j_start
   const uint2 *tile_table;  // [n_tiles] (row-block, col-block) of every tile of the launch (k_tile_table)
   const uint32_t *tc_ncnt;  // k_sweep_tc2<4>: per-sample N count over the swept words (k_tc_ncount), else null
-  unsigned long long *counter;
-  uint64_t *keys;
-  uint32_t *dvals;
-  unsigned long long cap;
+  union {
+    // thresholded sweeps: the edge list
+    struct {
+      unsigned long long *counter;
+      uint64_t *keys;
+      uint32_t *dvals;
+      unsigned long long cap;
+    };
+    // dense sweeps (k_sweep<true>, k_sweep_tc3<NP, true>): d(i, j) of every pair of the range is stored at
+    // dense[i * dense_ld + j - dense_col0], and with dense_mirror (square matrix) also at dense[j * dense_ld + i], plus an
+    // explicit 0 on the diagonal. No threshold, no list, no atomics. (A union: the struct keeps its size, and a larger
+    // parameter block changed the register allocation, and spills, of the existing tensor-core kernels.)
+    struct {
+      int32_t *dense;
+      uint64_t dense_ld;
+      uint32_t dense_col0;
+      uint32_t dense_mirror;
+    };
+  };
   uint32_t one;  // == 1, opaque to the compiler: acc += popc * one issues as IMAD on the FMA pipe
 };
 
@@ -693,6 +709,14 @@ static inline uint32_t tc_min_words() {
 static inline uint32_t next_window(uint32_t pw) { return pw < 8 ? 8 : pw < 16 ? 16 : (pw < PREFILTER_WORDS ? PREFILTER_WORDS : 0); }
 constexpr size_t SWEEP_SMEM = (size_t)STAGES * 2 * STAGE_U4 * sizeof(uint4);
 
+// The dynamic shared-memory array of every tile kernel of this file: its first declaration fixes the alignment for all
+// of them (128 B; the tensor-core kernels align their stages themselves). Declared here because k_sweep, a template,
+// is only instantiated after the tensor-core kernels, whose own declarations ask for 1024 B.
+extern __shared__ __align__(128) uint8_t smem_raw[];
+
+// DENSE: the epilogue stores every distance of the range (SweepArgs.dense) instead of thresholding and appending; a
+// template parameter, so that the thresholded instantiation compiles to the code it always had.
+template <bool DENSE>
 __global__ void __launch_bounds__(SWEEP_THREADS, 1) k_sweep(const SweepArgs a) {
   extern __shared__ __align__(128) uint8_t smem_raw[];
   uint4 *srow = reinterpret_cast<uint4 *>(smem_raw);       // [STAGES][KC][TILE]
@@ -822,6 +846,25 @@ __global__ void __launch_bounds__(SWEEP_THREADS, 1) k_sweep(const SweepArgs a) {
 
     // ---- epilogue: threshold + append -------------------------------------------------
     const uint32_t total_bits = a.Wp * 32u;
+    if constexpr (DENSE) {
+      // thread (tx, ty) holds rows rb*128 + i*16 + ty, cols cb*128 + j*16 + tx: the upper stores coalesce over tx, the
+      // mirror stores (square matrix) are scattered
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        const uint32_t gi = rb * TILE + i * 16 + ty;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const uint32_t gj = cb * TILE + j * 16 + tx;
+          if (gi < a.i_end && gj < a.n && gj > gi && gj >= a.j_start) {
+            const int32_t d = (int32_t)(total_bits - acc[i][j]);
+            a.dense[(uint64_t)gi * a.dense_ld + (gj - a.dense_col0)] = d;
+            if (a.dense_mirror) a.dense[(uint64_t)gj * a.dense_ld + gi] = d;
+          }
+        }
+        if (a.dense_mirror && cb == rb && tx == ty && gi < a.n) a.dense[(uint64_t)gi * a.dense_ld + gi] = 0;
+      }
+      continue;
+    }
     const uint32_t lane = tid & 31;
     // Most threads of a thresholded sweep hold no pair within the threshold (d = total_bits - matches): row maxima
     // of the 8 x 8 match counts decide that with ~70 instructions instead of ~15 per pair. A warp without any hit
@@ -1244,10 +1287,12 @@ namespace tracs {
 // One launch of the tile sweep over a.n_tiles tiles and a.Wp words: tensor-core kernel when the masks
 // allow its identity (no 2-/3-base codes at variable sites), LOP3/POPC kernel otherwise.
 // `has_n`: some variable site of some sample is N (ingest flag): the tensor-core kernel then needs its fourth plane.
-static void launch_tile_sweep(const SweepArgs &a_in, bool use_tc, cudaStream_t st, bool has_n = true) {
+// `dense`: the dense-output instantiations (k_sweep<true>, k_sweep_tc3<NP, true>) with a.dense set; TRACS_TC is ignored then.
+static void launch_tile_sweep(const SweepArgs &a_in, bool use_tc, cudaStream_t st, bool has_n = true, bool dense = false) {
   SweepArgs a = a_in;
   // the opt-in is per device (context): set on every call, it is a cheap driver call
-  TRACS_CK(cudaFuncSetAttribute(k_sweep, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SWEEP_SMEM));
+  TRACS_CK(cudaFuncSetAttribute(k_sweep<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SWEEP_SMEM));
+  TRACS_CK(cudaFuncSetAttribute(k_sweep<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SWEEP_SMEM));
   TRACS_CK(cudaFuncSetAttribute(k_sweep_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM));
   TRACS_CK(cudaFuncSetAttribute(k_sweep_tc2<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc2Geom<3>::SMEM));
   TRACS_CK(cudaFuncSetAttribute(k_sweep_tc2<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc2Geom<4>::SMEM));
@@ -1255,7 +1300,7 @@ static void launch_tile_sweep(const SweepArgs &a_in, bool use_tc, cudaStream_t s
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
   if (a.n_tiles == 0) return;
-  const char *tcv = getenv("TRACS_TC");  // "v1": the round-1 kernel (five one-hot planes), kept for comparison
+  const char *tcv = dense ? nullptr : getenv("TRACS_TC");  // "v1": the round-1 kernel (five one-hot planes), kept for comparison
   // which kernel ran: 10 * generation + operand planes executed (15 = k_sweep_tc, 23/24 = k_sweep_tc2, 33/34 = k_sweep_tc3)
   g_stats.tc_sweep = !use_tc ? 0.0f : (tcv && !strcmp(tcv, "v1")) ? 15.0f : ((tcv && !strcmp(tcv, "v2")) ? 20.0f : 30.0f) + (has_n ? 4.0f : 3.0f);
   DevBuf<uint32_t> ncnt;
@@ -1277,6 +1322,8 @@ static void launch_tile_sweep(const SweepArgs &a_in, bool use_tc, cudaStream_t s
       // 128 x 512 super-tiles: up to four consecutive tiles of a row-block share one expansion of the row panel
       TRACS_CK(cudaFuncSetAttribute(k_sweep_tc3<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc3Geom<3>::SMEM));
       TRACS_CK(cudaFuncSetAttribute(k_sweep_tc3<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc3Geom<4>::SMEM));
+      TRACS_CK(cudaFuncSetAttribute((k_sweep_tc3<3, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc3Geom<3>::SMEM));
+      TRACS_CK(cudaFuncSetAttribute((k_sweep_tc3<4, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc3Geom<4>::SMEM));
       std::vector<uint32_t> h_prefix(a.n_rb + 1), sprefix(a.n_rb + 1, 0);
       TRACS_CK(cudaMemcpyAsync(h_prefix.data(), a.tile_prefix, (a.n_rb + 1) * 4, cudaMemcpyDeviceToHost, st));
       TRACS_CK(cudaStreamSynchronize(st));
@@ -1290,14 +1337,18 @@ static void launch_tile_sweep(const SweepArgs &a_in, bool use_tc, cudaStream_t s
       const unsigned grid = (unsigned)std::min<uint64_t>(n_stiles, (uint64_t)n_sm);
       const char *dbg_env = getenv("TRACS_TC3_DBG");  // timing experiments (profiles/r2_tc.md); never set in production
       const uint32_t dbg = dbg_env ? (uint32_t)atoi(dbg_env) : 0u;
-      if (has_n) k_sweep_tc3<4><<<grid, TC3_THREADS, Tc3Geom<4>::SMEM, st>>>(a, d_stiles.p, n_stiles, dbg);
+      if (dense && has_n) k_sweep_tc3<4, true><<<grid, TC3_THREADS, Tc3Geom<4>::SMEM, st>>>(a, d_stiles.p, n_stiles, dbg);
+      else if (dense) k_sweep_tc3<3, true><<<grid, TC3_THREADS, Tc3Geom<3>::SMEM, st>>>(a, d_stiles.p, n_stiles, dbg);
+      else if (has_n) k_sweep_tc3<4><<<grid, TC3_THREADS, Tc3Geom<4>::SMEM, st>>>(a, d_stiles.p, n_stiles, dbg);
       else k_sweep_tc3<3><<<grid, TC3_THREADS, Tc3Geom<3>::SMEM, st>>>(a, d_stiles.p, n_stiles, dbg);
       TRACS_CK(cudaStreamSynchronize(st));  // sprefix (host) and the tables go out of scope
     }
   } else {
     int occ = 1;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_sweep, SWEEP_THREADS, SWEEP_SMEM);
-    k_sweep<<<(unsigned)std::min<uint64_t>(a.n_tiles, (uint64_t)n_sm * std::max(1, occ)), SWEEP_THREADS, SWEEP_SMEM, st>>>(a);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_sweep<false>, SWEEP_THREADS, SWEEP_SMEM);
+    const unsigned grid = (unsigned)std::min<uint64_t>(a.n_tiles, (uint64_t)n_sm * std::max(1, occ));
+    if (dense) k_sweep<true><<<grid, SWEEP_THREADS, SWEEP_SMEM, st>>>(a);
+    else k_sweep<false><<<grid, SWEEP_THREADS, SWEEP_SMEM, st>>>(a);
   }
   g_stats.kernel_launches++;
   TRACS_CK(cudaGetLastError());
@@ -1640,6 +1691,29 @@ static TilePlan plan_tiles(uint64_t n, uint64_t i_end, uint64_t j_start, uint32_
   return p;
 }
 
+// Consecutive row-blocks of a plan cut into bands of at most `limit` pairs and `tile_limit` tiles (one launch each):
+// my_rb[first, last).
+struct Band { size_t first, last; uint64_t pairs; };
+constexpr uint64_t BAND_PAIRS = 1ull << 28;  // pairs per band of a full-length sweep (the edge buffer holds every pair of one)
+static std::vector<Band> make_bands(const TilePlan &plan, uint64_t limit, uint64_t tile_limit) {
+  std::vector<Band> u;
+  size_t b0 = 0;
+  uint64_t acc = 0, tiles = 0;
+  for (size_t k = 0; k < plan.my_rb.size(); ++k) {
+    const uint64_t p = plan.rb_pairs[k], t = plan.n_cb - std::max(plan.my_rb[k], plan.cb_min);
+    if (k > b0 && (acc + p > limit || tiles + t > tile_limit)) {
+      u.push_back({b0, k, acc});
+      b0 = k;
+      acc = 0;
+      tiles = 0;
+    }
+    acc += p;
+    tiles += t;
+  }
+  if (b0 < plan.my_rb.size()) u.push_back({b0, plan.my_rb.size(), acc});
+  return u;
+}
+
 }  // namespace tracs
 #include "pairs.inl"
 namespace tracs {
@@ -1678,32 +1752,15 @@ void sweep_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint64_t pitc
   // candidate list is bounded (CAND_CAP) because only a few per cent of the pairs may survive. Otherwise, or when the
   // prefilter is not selective, the row-blocks are cut into bands whose pair count fits the edge buffer (a full-length
   // sweep may emit every pair).
-  struct Unit { size_t first, last; uint64_t pairs; };
-  const uint64_t CAP_MAX = 1ull << 28, CAND_CAP = 1ull << 26;
+  using Unit = Band;
+  const uint64_t CAP_MAX = BAND_PAIRS, CAND_CAP = 1ull << 26;
   uint64_t total_pairs = 0, total_tiles = 0;
   for (size_t k = 0; k < my_rb.size(); ++k) {
     total_pairs += plan.rb_pairs[k];
     total_tiles += n_cb - std::max(my_rb[k], cb_min);
   }
   S.n_pairs += total_pairs;
-  auto make_units = [&](uint64_t limit, uint64_t tile_limit) {
-    std::vector<Unit> u;
-    size_t b0 = 0;
-    uint64_t acc = 0, tiles = 0;
-    for (size_t k = 0; k < my_rb.size(); ++k) {
-      const uint64_t p = plan.rb_pairs[k], t = n_cb - std::max(my_rb[k], cb_min);
-      if (k > b0 && (acc + p > limit || tiles + t > tile_limit)) {
-        u.push_back({b0, k, acc});
-        b0 = k;
-        acc = 0;
-        tiles = 0;
-      }
-      acc += p;
-      tiles += t;
-    }
-    if (b0 < my_rb.size()) u.push_back({b0, my_rb.size(), acc});
-    return u;
-  };
+  auto make_units = [&](uint64_t limit, uint64_t tile_limit) { return make_bands(plan, limit, tile_limit); };
   if (my_rb.empty()) {
     S.ms_total = Ttot.stop();
     return;
@@ -2008,6 +2065,60 @@ void sweep_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint64_t pitc
   if (!fall_back) break;
   prefilter_mode = false;  // second pass: banded full-length sweeps
   }
+  S.ms_total = Ttot.stop();
+}
+
+// All-pairs distances of the device-resident alignment as a dense int32 matrix (tracs_distance_matrix_device): the
+// ingest, the tile plan and the full-length tile sweep of sweep_device, with the dense epilogue instead of threshold,
+// list, sort and compared sites. Square (o.i_end == n, o.j_start == 0): out[i][j] = out[j][i] = d(i, j), zero diagonal.
+// Rectangle (o.j_start >= o.i_end): out[i][j - j_start] for i < i_end <= j_start <= j < n. Arguments validated by the caller.
+void distance_matrix_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint64_t pitch, const tracs_opts_t &o, int32_t *out,
+                            uint64_t ld, cudaStream_t st) {
+  tracs_stats_t &S = g_stats;
+  S.n_samples = n;
+  S.seq_length = L;
+  const uint64_t i_end = std::min<uint64_t>(o.i_end, n), j_start = o.j_start;
+  if (n == 0 || i_end == 0 || j_start >= n) return;
+  if (n >= (1ull << 31)) throw std::runtime_error("too many samples");
+  const bool square = j_start == 0;
+  Timer T(st), Ttot(st);
+  Ttot.start();
+  Ingested ing;
+  ingest_device(dev_seqs, n, L, pitch, o.packed_input != 0, false, ing, st);
+  if (o.sweep_variant == 2 && ing.partial_ambiguity)
+    throw std::runtime_error("tensor-core sweep requested but the alignment has 2-/3-base IUPAC codes at variable sites");
+  const bool use_tc = o.sweep_variant != 1 && !ing.partial_ambiguity;
+  const TilePlan plan = plan_tiles(n, i_end, j_start, ing.Npad, 0, 1);
+  // bands as on the sparse path: one launch each, Ctrl-C is seen between them
+  const std::vector<Band> bands = make_bands(plan, BAND_PAIRS, 1ull << 31);
+  DevBuf<uint32_t> d_rb(std::max<size_t>(1, plan.my_rb.size())), d_prefix(plan.my_rb.size() + 1);
+  for (const Band &b : bands) {
+    check_interrupt();
+    std::vector<uint32_t> rbs(plan.my_rb.begin() + b.first, plan.my_rb.begin() + b.last);
+    std::vector<uint32_t> prefix(rbs.size() + 1, 0);
+    for (size_t k = 0; k < rbs.size(); ++k) prefix[k + 1] = prefix[k] + (plan.n_cb - std::max(rbs[k], plan.cb_min));
+    const uint32_t n_tiles = prefix.back();
+    TRACS_CK(cudaMemcpyAsync(d_rb.p, rbs.data(), rbs.size() * 4, cudaMemcpyHostToDevice, st));
+    TRACS_CK(cudaMemcpyAsync(d_prefix.p, prefix.data(), prefix.size() * 4, cudaMemcpyHostToDevice, st));
+    SweepArgs a;
+    a.planes = ing.planes.p; a.Wp = ing.Wp; a.Npad = ing.Npad; a.n = (uint32_t)n; a.i_end = (uint32_t)i_end;
+    a.j_start = (uint32_t)j_start; a.dist = INT32_MAX; a.rb_list = d_rb.p; a.tile_prefix = d_prefix.p;
+    a.n_rb = (uint32_t)rbs.size(); a.n_tiles = n_tiles; a.cb_min = plan.cb_min; a.one = 1; a.tc_ncnt = nullptr;
+    a.dense = out; a.dense_ld = ld; a.dense_col0 = (uint32_t)j_start; a.dense_mirror = square ? 1u : 0u;
+    DevBuf<uint2> d_table(std::max<uint32_t>(1, n_tiles));
+    if (n_tiles) {
+      k_tile_table<<<(n_tiles + 255) / 256, 256, 0, st>>>(d_rb.p, d_prefix.p, a.n_rb, plan.cb_min, n_tiles, d_table.p);
+      S.kernel_launches++;
+    }
+    a.tile_table = d_table.p;
+    T.start();
+    launch_tile_sweep(a, use_tc, st, ing.has_n_var, true);
+    S.ms_sweep += T.stop();
+    S.n_tiles += n_tiles;
+    S.n_pairs += b.pairs;
+    S.swept_wordpairs += b.pairs * std::max<uint64_t>(ing.W, 1);
+  }
+  TRACS_CK(cudaStreamSynchronize(st));
   S.ms_total = Ttot.stop();
 }
 
