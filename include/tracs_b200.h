@@ -75,8 +75,8 @@ typedef struct tracs_stats {
   float ms_total;            /* device time of the whole call (events on the call's stream) */
   float ms_d2h;              /* edge columns device -> host                                  */
   float ms_filter;           /* recombination filter (K4), only when filter != 0             */
-  float tc_sweep;            /* 0: LOP3/POPC tile kernel; else 10 * generation + int8 operand planes executed per site:
-                                15 = k_sweep_tc, 23 / 24 = k_sweep_tc2<3|4>, 33 / 34 = k_sweep_tc3<3|4> */
+  float tc_sweep;            /* 0: LOP3/POPC tile kernel; else 30 + int8 operand planes executed per site:
+                                33 / 34 = k_sweep_tc3<3|4> */
   float ms_pack_main;        /* the main pack launch alone: k_pack_x over samples 256.. (early extraction) or k_pack over all */
   float sparse_nplane;       /* 1: sparse N (first-chunk estimate): the main ingest launch stored only the N-plane sectors that hold an N */
   float reserved0;
@@ -290,7 +290,7 @@ int tracs_int_peak(double out[8]);
 
 /* Measures the int8 tensor-pipe peak on the current device: every SM issues back-to-back
  * tcgen05.mma.cta_group::1.kind::i8 (M = 128, K = 32) from shared-memory operands into TMEM.
- * out[0] = TOP/s with N = 128 (the shape k_sweep_tc issues), out[1] = TOP/s with N = 256,
+ * out[0] = TOP/s with N = 128 (one 128 x 128 tile per MMA), out[1] = TOP/s with N = 256 (the shape k_sweep_tc3 issues),
  * out[2], out[3] = SM clock cycles per MMA for the two shapes. */
 int tracs_tc_peak(double out[4]);
 /* The same probe held for `seconds` (0.05 .. 10): out[0] = TOP/s over the second half of the run (what the pipe sustains under

@@ -382,7 +382,7 @@ def test_tensor_core_sweep_modes(oracle_mod):
     for n1 in (100, 300):
         res = tracs_b200.pairsnp_matrix(s, dist=200, i_end=n1, j_start=n1, full_sweep="tc")
         _cmp(res, oracle_mod.pairsnp_ascii(s, i_end=n1, j_start=n1, dist=200, n_threads=4))
-    full = tracs_b200.pairsnp_matrix(s, dist=IMAX)            # auto: no prefilter possible -> k_sweep_tc
+    full = tracs_b200.pairsnp_matrix(s, dist=IMAX)            # auto: no prefilter possible -> k_sweep_tc3
     _cmp(full, oracle_mod.pairsnp_ascii(s, dist=IMAX, n_threads=4))
     pop = tracs_b200.pairsnp_matrix(s, dist=IMAX, full_sweep=True)   # forced LOP3/POPC kernel
     for k in ("rows", "cols", "dist", "ncomp"):
@@ -424,19 +424,14 @@ def test_filter_decisions_match_incomplete_beta_cdf():
 
 @pytest.mark.parametrize("n,L,dist,p_N", [(100, 3000, IMAX, 0.0), (300, 20000, 30, 0.0), (513, 9000, IMAX, 0.0), (257, 33000, 500, 0.2),
                                           (130, 70001, IMAX, 0.01), (1100, 6000, 40, 0.0), (900, 5000, 60, 0.05)])
-def test_tensor_core_sweep_v2_planes(oracle_mod, monkeypatch, n, L, dist, p_N):
-    """k_sweep_tc2: three +-1 planes when no variable site holds an N (NP = 3), plus the N plane and the per-sample N
-    counts otherwise (NP = 4); against the oracle and against the round-1 kernel (TRACS_TC=v1)."""
+def test_tensor_core_sweep_planes(oracle_mod, n, L, dist, p_N):
+    """k_sweep_tc3: three +-1 planes when no variable site holds an N (NP = 3), plus the N plane and the per-sample N
+    counts otherwise (NP = 4); against the oracle."""
     s = synth.generate(n, L, p_var=0.08, n_clusters=5, mu=4, p_N=p_N, p_amb=0.0, seed=n + L, lowercase=0.05, gaps=0 if p_N == 0 else 2)
     orc = oracle_mod.pairsnp_ascii(s, dist=dist, n_threads=4)
     res = tracs_b200.pairsnp_matrix(s, dist=dist, full_sweep="tc")      # k_sweep_tc3: 128 x 512 super-tiles
     assert tracs_b200.last_stats()["tc_sweep"] in (33.0, 34.0)          # generation 3, three or four operand planes
     _cmp(res, orc)
-    for v, codes in (("v2", (23.0, 24.0)), ("v1", (15.0,))):             # 128 x 128 tiles; the round-1 kernel
-        monkeypatch.setenv("TRACS_TC", v)
-        _cmp(tracs_b200.pairsnp_matrix(s, dist=dist, full_sweep="tc"), orc)
-        assert tracs_b200.last_stats()["tc_sweep"] in codes
-    monkeypatch.delenv("TRACS_TC")
     for n1 in (n // 3, n - 1):                                           # query x db ranges cut super-tiles short
         _cmp(tracs_b200.pairsnp_matrix(s, dist=dist, i_end=n1, j_start=n1, full_sweep="tc"),
              oracle_mod.pairsnp_ascii(s, i_end=n1, j_start=n1, dist=dist, n_threads=4))

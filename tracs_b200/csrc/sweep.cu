@@ -450,7 +450,7 @@ k_gather(const uint8_t *__restrict__ seqs, uint64_t n, uint64_t pitch, const uin
       const uint64_t s = sb + t;
       if (s >= s1) break;
       const uint32_t m = mk[t];
-      // two- or three-base codes at a variable site rule out the one-hot GEMM identity (sweep_tc.inl)
+      // two- or three-base codes at a variable site rule out the tensor-core identity (sweep_tc3.inl)
       if (__any_sync(0xFFFFFFFFu, m != 15u && (m & (m - 1)) != 0u) && lane == 0) atomicOr(amb_flag, 1u);
       if (__any_sync(0xFFFFFFFFu, live && m == 15u) && lane == 0) atomicOr(amb_flag, 2u);  // an N at a variable site
       const uint32_t A = __ballot_sync(0xFFFFFFFFu, m & 1);
@@ -618,7 +618,7 @@ struct SweepArgs {
   uint32_t n_tiles;
   uint32_t cb_min;  // first col-block allowed by j_start
   const uint2 *tile_table;  // [n_tiles] (row-block, col-block) of every tile of the launch (k_tile_table)
-  const uint32_t *tc_ncnt;  // k_sweep_tc2<4>: per-sample N count over the swept words (k_tc_ncount), else null
+  const uint32_t *tc_ncnt;  // k_sweep_tc3<4>: per-sample N count over the swept words (k_tc_ncount), else null
   union {
     // thresholded sweeps: the edge list
     struct {
@@ -701,11 +701,8 @@ static inline uint32_t first_window(int64_t dist) {
   if (dist < 43) return 8;
   return prefilter_words(dist);
 }
-// narrowest prefilter window that goes to the tensor-core kernel when the masks allow it (TRACS_TC_MIN_WORDS: experiments)
-static inline uint32_t tc_min_words() {
-  const char *e = getenv("TRACS_TC_MIN_WORDS");
-  return e ? (uint32_t)atoi(e) : 17u;
-}
+// narrowest prefilter window that goes to the tensor-core kernel when the masks allow it (DESIGN.md section 7)
+constexpr uint32_t TC_MIN_WORDS = 17;
 static inline uint32_t next_window(uint32_t pw) { return pw < 8 ? 8 : pw < 16 ? 16 : (pw < PREFILTER_WORDS ? PREFILTER_WORDS : 0); }
 constexpr size_t SWEEP_SMEM = (size_t)STAGES * 2 * STAGE_U4 * sizeof(uint4);
 
@@ -1279,34 +1276,26 @@ __global__ void k_trans_gather(const uint64_t *__restrict__ keys, const uint32_t
 }
 
 }  // namespace tracs
-#include "sweep_tc.inl"
-#include "sweep_tc2.inl"
 #include "sweep_tc3.inl"
 namespace tracs {
 
 // One launch of the tile sweep over a.n_tiles tiles and a.Wp words: tensor-core kernel when the masks
 // allow its identity (no 2-/3-base codes at variable sites), LOP3/POPC kernel otherwise.
 // `has_n`: some variable site of some sample is N (ingest flag): the tensor-core kernel then needs its fourth plane.
-// `dense`: the dense-output instantiations (k_sweep<true>, k_sweep_tc3<NP, true>) with a.dense set; TRACS_TC is ignored then.
-static void launch_tile_sweep(const SweepArgs &a_in, bool use_tc, cudaStream_t st, bool has_n = true, bool dense = false) {
+// `dense`: the dense-output instantiations (k_sweep<true>, k_sweep_tc3<NP, true>) with a.dense set.
+static void launch_tile_sweep(const SweepArgs &a_in, bool use_tc, cudaStream_t st, bool has_n, bool dense) {
   SweepArgs a = a_in;
   // the opt-in is per device (context): set on every call, it is a cheap driver call
   TRACS_CK(cudaFuncSetAttribute(k_sweep<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SWEEP_SMEM));
   TRACS_CK(cudaFuncSetAttribute(k_sweep<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SWEEP_SMEM));
-  TRACS_CK(cudaFuncSetAttribute(k_sweep_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM));
-  TRACS_CK(cudaFuncSetAttribute(k_sweep_tc2<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc2Geom<3>::SMEM));
-  TRACS_CK(cudaFuncSetAttribute(k_sweep_tc2<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc2Geom<4>::SMEM));
   int dev = 0, n_sm = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
   if (a.n_tiles == 0) return;
-  const char *tcv = dense ? nullptr : getenv("TRACS_TC");  // "v1": the round-1 kernel (five one-hot planes), kept for comparison
-  // which kernel ran: 10 * generation + operand planes executed (15 = k_sweep_tc, 23/24 = k_sweep_tc2, 33/34 = k_sweep_tc3)
-  g_stats.tc_sweep = !use_tc ? 0.0f : (tcv && !strcmp(tcv, "v1")) ? 15.0f : ((tcv && !strcmp(tcv, "v2")) ? 20.0f : 30.0f) + (has_n ? 4.0f : 3.0f);
-  DevBuf<uint32_t> ncnt;
-  if (use_tc && tcv && !strcmp(tcv, "v1")) {
-    k_sweep_tc<<<(unsigned)std::min<uint64_t>(a.n_tiles, (uint64_t)n_sm), TC_THREADS, TC_SMEM, st>>>(a);
-  } else if (use_tc) {
+  // which kernel ran: 0 = k_sweep, else 30 + operand planes executed (33/34 = k_sweep_tc3<3|4>)
+  g_stats.tc_sweep = use_tc ? 30.0f + (has_n ? 4.0f : 3.0f) : 0.0f;
+  if (use_tc) {
+    DevBuf<uint32_t> ncnt;
     a.tc_ncnt = nullptr;
     if (has_n) {
       ncnt.alloc(a.Npad);
@@ -1314,35 +1303,29 @@ static void launch_tile_sweep(const SweepArgs &a_in, bool use_tc, cudaStream_t s
       g_stats.kernel_launches++;
       a.tc_ncnt = ncnt.p;
     }
-    if (tcv && !strcmp(tcv, "v2")) {  // 128 x 128 tiles (kept for comparison)
-      const unsigned grid = (unsigned)std::min<uint64_t>(a.n_tiles, (uint64_t)n_sm);
-      if (has_n) k_sweep_tc2<4><<<grid, TC2_THREADS, Tc2Geom<4>::SMEM, st>>>(a);
-      else k_sweep_tc2<3><<<grid, TC2_THREADS, Tc2Geom<3>::SMEM, st>>>(a);
-    } else {
-      // 128 x 512 super-tiles: up to four consecutive tiles of a row-block share one expansion of the row panel
-      TRACS_CK(cudaFuncSetAttribute(k_sweep_tc3<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc3Geom<3>::SMEM));
-      TRACS_CK(cudaFuncSetAttribute(k_sweep_tc3<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc3Geom<4>::SMEM));
-      TRACS_CK(cudaFuncSetAttribute((k_sweep_tc3<3, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc3Geom<3>::SMEM));
-      TRACS_CK(cudaFuncSetAttribute((k_sweep_tc3<4, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc3Geom<4>::SMEM));
-      std::vector<uint32_t> h_prefix(a.n_rb + 1), sprefix(a.n_rb + 1, 0);
-      TRACS_CK(cudaMemcpyAsync(h_prefix.data(), a.tile_prefix, (a.n_rb + 1) * 4, cudaMemcpyDeviceToHost, st));
-      TRACS_CK(cudaStreamSynchronize(st));
-      for (uint32_t k = 0; k < a.n_rb; ++k) sprefix[k + 1] = sprefix[k] + (h_prefix[k + 1] - h_prefix[k] + 3) / 4;
-      const uint32_t n_stiles = sprefix[a.n_rb];
-      DevBuf<uint32_t> d_sprefix(a.n_rb + 1);
-      DevBuf<uint2> d_stiles(std::max<uint32_t>(1, n_stiles));
-      TRACS_CK(cudaMemcpyAsync(d_sprefix.p, sprefix.data(), (a.n_rb + 1) * 4, cudaMemcpyHostToDevice, st));
-      k_stile_table<<<(n_stiles + 255) / 256, 256, 0, st>>>(a.rb_list, d_sprefix.p, a.n_rb, a.cb_min, a.Npad / TILE, n_stiles, d_stiles.p);
-      g_stats.kernel_launches++;
-      const unsigned grid = (unsigned)std::min<uint64_t>(n_stiles, (uint64_t)n_sm);
-      const char *dbg_env = getenv("TRACS_TC3_DBG");  // timing experiments (profiles/r2_tc.md); never set in production
-      const uint32_t dbg = dbg_env ? (uint32_t)atoi(dbg_env) : 0u;
-      if (dense && has_n) k_sweep_tc3<4, true><<<grid, TC3_THREADS, Tc3Geom<4>::SMEM, st>>>(a, d_stiles.p, n_stiles, dbg);
-      else if (dense) k_sweep_tc3<3, true><<<grid, TC3_THREADS, Tc3Geom<3>::SMEM, st>>>(a, d_stiles.p, n_stiles, dbg);
-      else if (has_n) k_sweep_tc3<4><<<grid, TC3_THREADS, Tc3Geom<4>::SMEM, st>>>(a, d_stiles.p, n_stiles, dbg);
-      else k_sweep_tc3<3><<<grid, TC3_THREADS, Tc3Geom<3>::SMEM, st>>>(a, d_stiles.p, n_stiles, dbg);
-      TRACS_CK(cudaStreamSynchronize(st));  // sprefix (host) and the tables go out of scope
-    }
+    // 128 x 512 super-tiles: up to four consecutive tiles of a row-block share one expansion of the row panel
+    TRACS_CK(cudaFuncSetAttribute(k_sweep_tc3<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc3Geom<3>::SMEM));
+    TRACS_CK(cudaFuncSetAttribute(k_sweep_tc3<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc3Geom<4>::SMEM));
+    TRACS_CK(cudaFuncSetAttribute((k_sweep_tc3<3, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc3Geom<3>::SMEM));
+    TRACS_CK(cudaFuncSetAttribute((k_sweep_tc3<4, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc3Geom<4>::SMEM));
+    std::vector<uint32_t> h_prefix(a.n_rb + 1), sprefix(a.n_rb + 1, 0);
+    TRACS_CK(cudaMemcpyAsync(h_prefix.data(), a.tile_prefix, (a.n_rb + 1) * 4, cudaMemcpyDeviceToHost, st));
+    TRACS_CK(cudaStreamSynchronize(st));
+    for (uint32_t k = 0; k < a.n_rb; ++k) sprefix[k + 1] = sprefix[k] + (h_prefix[k + 1] - h_prefix[k] + 3) / 4;
+    const uint32_t n_stiles = sprefix[a.n_rb];
+    DevBuf<uint32_t> d_sprefix(a.n_rb + 1);
+    DevBuf<uint2> d_stiles(std::max<uint32_t>(1, n_stiles));
+    TRACS_CK(cudaMemcpyAsync(d_sprefix.p, sprefix.data(), (a.n_rb + 1) * 4, cudaMemcpyHostToDevice, st));
+    k_stile_table<<<(n_stiles + 255) / 256, 256, 0, st>>>(a.rb_list, d_sprefix.p, a.n_rb, a.cb_min, a.Npad / TILE, n_stiles, d_stiles.p);
+    g_stats.kernel_launches++;
+    const unsigned grid = (unsigned)std::min<uint64_t>(n_stiles, (uint64_t)n_sm);
+    const char *dbg_env = getenv("TRACS_TC3_DBG");  // timing experiments (profiles/r2_tc.md); never set in production
+    const uint32_t dbg = dbg_env ? (uint32_t)atoi(dbg_env) : 0u;
+    if (dense && has_n) k_sweep_tc3<4, true><<<grid, TC3_THREADS, Tc3Geom<4>::SMEM, st>>>(a, d_stiles.p, n_stiles, dbg);
+    else if (dense) k_sweep_tc3<3, true><<<grid, TC3_THREADS, Tc3Geom<3>::SMEM, st>>>(a, d_stiles.p, n_stiles, dbg);
+    else if (has_n) k_sweep_tc3<4><<<grid, TC3_THREADS, Tc3Geom<4>::SMEM, st>>>(a, d_stiles.p, n_stiles, dbg);
+    else k_sweep_tc3<3><<<grid, TC3_THREADS, Tc3Geom<3>::SMEM, st>>>(a, d_stiles.p, n_stiles, dbg);
+    TRACS_CK(cudaStreamSynchronize(st));  // sprefix (host) and the tables go out of scope
   } else {
     int occ = 1;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_sweep<false>, SWEEP_THREADS, SWEEP_SMEM);
@@ -1695,6 +1678,8 @@ static TilePlan plan_tiles(uint64_t n, uint64_t i_end, uint64_t j_start, uint32_
 // my_rb[first, last).
 struct Band { size_t first, last; uint64_t pairs; };
 constexpr uint64_t BAND_PAIRS = 1ull << 28;  // pairs per band of a full-length sweep (the edge buffer holds every pair of one)
+constexpr uint64_t BAND_TILES = 1ull << 31;  // tiles per launch (the kernels count tiles in 32 bits)
+constexpr uint64_t CAND_CAP = 1ull << 26;    // prefilter candidates held at once (only a few per cent of the pairs may survive)
 static std::vector<Band> make_bands(const TilePlan &plan, uint64_t limit, uint64_t tile_limit) {
   std::vector<Band> u;
   size_t b0 = 0;
@@ -1714,12 +1699,390 @@ static std::vector<Band> make_bands(const TilePlan &plan, uint64_t limit, uint64
   return u;
 }
 
+// radix-sort end bit of the pair keys (i << 32 | j), i, j < n
+static int key_end_bit(uint64_t n) {
+  int end_bit = 32;
+  while ((1ull << (end_bit - 32)) < n) end_bit++;
+  return end_bit;
+}
+
+// Tensor cores unless forced off (sweep_variant 1) or inapplicable (2-/3-base codes at variable sites); sweep_variant 2
+// insists on them.
+static bool use_tensor_cores(const tracs_opts_t &o, const Ingested &g) {
+  if (o.sweep_variant == 2 && g.partial_ambiguity)
+    throw std::runtime_error("tensor-core sweep requested but the alignment has 2-/3-base IUPAC codes at variable sites");
+  return o.sweep_variant != 1 && !g.partial_ambiguity;
+}
+
+// The fields every tile sweep of an ingested alignment shares; the caller adds the output (edge list or dense matrix),
+// sweep_band() the tile list.
+static SweepArgs sweep_args(const Ingested &g, uint64_t i_end, uint64_t j_start, int32_t dist) {
+  SweepArgs a{};
+  a.planes = g.planes.p; a.Wp = g.Wp; a.Npad = g.Npad; a.n = (uint32_t)g.n; a.i_end = (uint32_t)i_end;
+  a.j_start = (uint32_t)j_start; a.dist = dist; a.one = 1;
+  return a;
+}
+
+// One launch of the tile sweep over the row-blocks plan.my_rb[b.first, b.last): the tile list (prefix, copies,
+// k_tile_table), the launch on `a` (planes, window, range and output already set) and its stats. Returns the tile count.
+static uint32_t sweep_band(const TilePlan &plan, const Band &b, SweepArgs a, bool use_tc, bool has_n, bool dense, cudaStream_t st) {
+  tracs_stats_t &S = g_stats;
+  const std::vector<uint32_t> rbs(plan.my_rb.begin() + b.first, plan.my_rb.begin() + b.last);
+  std::vector<uint32_t> prefix(rbs.size() + 1, 0);
+  for (size_t k = 0; k < rbs.size(); ++k) prefix[k + 1] = prefix[k] + (plan.n_cb - std::max(rbs[k], plan.cb_min));
+  const uint32_t n_tiles = prefix.back();
+  DevBuf<uint32_t> d_rb(std::max<size_t>(1, rbs.size())), d_prefix(prefix.size());
+  DevBuf<uint2> d_table(std::max<uint32_t>(1, n_tiles));
+  TRACS_CK(cudaMemcpyAsync(d_rb.p, rbs.data(), rbs.size() * 4, cudaMemcpyHostToDevice, st));
+  TRACS_CK(cudaMemcpyAsync(d_prefix.p, prefix.data(), prefix.size() * 4, cudaMemcpyHostToDevice, st));
+  a.rb_list = d_rb.p; a.tile_prefix = d_prefix.p; a.n_rb = (uint32_t)rbs.size(); a.n_tiles = n_tiles; a.cb_min = plan.cb_min;
+  a.tile_table = d_table.p;
+  if (n_tiles) {
+    k_tile_table<<<(n_tiles + 255) / 256, 256, 0, st>>>(d_rb.p, d_prefix.p, a.n_rb, plan.cb_min, n_tiles, d_table.p);
+    S.kernel_launches++;
+  }
+  Timer T(st);
+  T.start();
+  launch_tile_sweep(a, use_tc, st, has_n, dense);
+  S.ms_sweep += T.stop();
+  S.n_tiles += n_tiles;
+  return n_tiles;
+}
+
+// Edge (or candidate) list of a thresholded sweep: the tile kernels append (key, distance) pairs through `counter`; the
+// second pair of buffers receives sorts and compactions.
+struct EdgeList {
+  uint64_t cap;
+  DevBuf<uint64_t> keys, keys2;
+  DevBuf<uint32_t> dv, dv2;
+  DevBuf<unsigned long long> counter;
+  explicit EdgeList(uint64_t c) : cap(c), keys(c), keys2(c), dv(c), dv2(c), counter(1) {}
+  void output_to(SweepArgs &a) const { a.counter = counter.p; a.keys = keys.p; a.dvals = dv.p; a.cap = cap; }
+  void reset(cudaStream_t st) { TRACS_CK(cudaMemsetAsync(counter.p, 0, sizeof(unsigned long long), st)); }
+  uint64_t count(cudaStream_t st) const {
+    unsigned long long c = 0;
+    TRACS_CK(cudaMemcpyAsync(&c, counter.p, sizeof c, cudaMemcpyDeviceToHost, st));
+    TRACS_CK(cudaStreamSynchronize(st));
+    return c;
+  }
+  void swap() {  // (keys2, dv2) become the current list
+    std::swap(keys.p, keys2.p);
+    std::swap(dv.p, dv2.p);
+  }
+};
+
+// Filter-and-refine, first step: tile-sweep only the first words of every pair of the plan into `c`; d is monotone in
+// the number of sites, so a pair whose partial distance already exceeds a.dist is decided. Windows of 4, 8, 16 and 64
+// words (at most the ingested words) are tried in turn until the candidates fit the list and are <= 4 % of `pairs` --
+// per-pair refinement is then cheaper than tiles -- or the widest window has been swept. A narrow window (< 16 words)
+// lets a few unrelated pairs through; left in, they would bridge clusters in the candidate graph, so its candidates are
+// trimmed over the next words (k_cand_trim). Short windows run on the LOP3/POPC kernel (the tensor-core kernel pays its
+// per-tile pipeline fill and its TMEM epilogue on every 128 x 128 tile: measured equal at 16 words, slower below), wider
+// ones on the tensor cores when `tc_ok`. The candidates are left unsorted in (c.keys, c.dv).
+struct Prefilter {
+  uint64_t n_cand;
+  uint32_t words;   // window that produced the candidates
+  bool selective;   // they fit the list and are <= 4 % of the pairs
+};
+static Prefilter prefilter(const Ingested &g, const TilePlan &plan, uint64_t pairs, SweepArgs a, bool tc_ok, EdgeList &c,
+                           cudaStream_t st) {
+  tracs_stats_t &S = g_stats;
+  const std::vector<Band> bands = make_bands(plan, UINT64_MAX, BAND_TILES);
+  c.output_to(a);
+  for (uint32_t pw = first_window(a.dist);; pw = next_window(pw)) {
+    const uint32_t words = std::min(pw, g.Wp);
+    a.Wp = words;
+    c.reset(st);
+    for (const Band &b : bands) sweep_band(plan, b, a, tc_ok && words >= TC_MIN_WORDS, g.has_n_var, false, st);
+    S.swept_wordpairs += pairs * words;
+    uint64_t n_cand = c.count(st);
+    const bool selective = n_cand <= c.cap && n_cand * 25 <= pairs;
+    if (selective && n_cand && words < 16 && g.Wp > words) {
+      Timer T(st);
+      T.start();
+      const uint32_t extra = std::min<uint32_t>(g.Wp - words, 32 - words);
+      DevBuf<uint8_t> flags(n_cand);
+      DevBuf<uint64_t> n_sel(1);
+      k_cand_trim<<<(unsigned)((n_cand + 255) / 256), 256, 0, st>>>(c.keys.p, c.dv.p, n_cand, g.planesT.p, g.Wp, words, extra, a.dist,
+                                                                     flags.p);
+      size_t tb = 0;
+      cub::DeviceSelect::Flagged(nullptr, tb, c.keys.p, flags.p, c.keys2.p, n_sel.p, (int64_t)n_cand, st);
+      DevBuf<uint8_t> tmp(tb);
+      cub::DeviceSelect::Flagged(tmp.p, tb, c.keys.p, flags.p, c.keys2.p, n_sel.p, (int64_t)n_cand, st);
+      cub::DeviceSelect::Flagged(tmp.p, tb, c.dv.p, flags.p, c.dv2.p, n_sel.p, (int64_t)n_cand, st);
+      TRACS_CK(cudaMemcpyAsync(&n_cand, n_sel.p, 8, cudaMemcpyDeviceToHost, st));
+      TRACS_CK(cudaStreamSynchronize(st));
+      c.swap();
+      S.kernel_launches += 5;
+      S.ms_refine += T.stop();
+    }
+    if (selective || words >= std::min(PREFILTER_WORDS, g.Wp)) {
+      S.n_candidates += n_cand;
+      return {n_cand, words, selective};
+    }
+  }
+}
+
+// Where E new rows of an edge table start in each of its columns; null: the column is not filled.
+struct HostColumns {
+  uint64_t *rows, *cols, *dist, *ncomp, *filt;
+  double *p0_log, *eK, *datediff;
+};
+// Appends E rows to the columns of `out` that the call fills (rows, cols, dist always; compared sites, filtered distance and
+// the likelihood columns when asked for) and returns where they start.
+static HostColumns append_rows(HostEdges &out, uint64_t E, bool ncomp, bool filt, bool trans) {
+  const size_t old = out.rows.size();
+  out.rows.resize(old + E); out.cols.resize(old + E); out.dist.resize(old + E);
+  if (ncomp) out.ncomp.resize(old + E);
+  if (filt) out.filt.resize(old + E);
+  if (trans) { out.p0_log.resize(old + E); out.eK.resize(old + E); out.datediff.resize(old + E); }
+  return {out.rows.data() + old, out.cols.data() + old, out.dist.data() + old, ncomp ? out.ncomp.data() + old : nullptr,
+          filt ? out.filt.data() + old : nullptr, trans ? out.p0_log.data() + old : nullptr, trans ? out.eK.data() + old : nullptr,
+          trans ? out.datediff.data() + old : nullptr};
+}
+// Enqueues the device -> host copies of E rows of every column that `src` (device) gives into the same column of `dst`.
+static void copy_columns(const HostColumns &dst, const HostColumns &src, uint64_t E, cudaStream_t st) {
+  auto copy = [&](void *d, const void *s) {
+    if (!s) return;
+    TRACS_CK(cudaMemcpyAsync(d, s, E * 8, cudaMemcpyDeviceToHost, st));
+    g_stats.d2h_bytes += E * 8;
+  };
+  copy(dst.rows, src.rows); copy(dst.cols, src.cols); copy(dst.dist, src.dist); copy(dst.ncomp, src.ncomp); copy(dst.filt, src.filt);
+  copy(dst.p0_log, src.p0_log); copy(dst.eK, src.eK); copy(dst.datediff, src.datediff);
+}
+
+// Two events that order the auxiliary stream against the main one, per host thread and device (an event belongs to the
+// device it was created on, and a thread may drive several).
+struct AuxEvents { cudaEvent_t a, b; };
+static AuxEvents aux_events() {
+  static thread_local AuxEvents ev[64] = {};
+  int dev = 0;
+  TRACS_CK(cudaGetDevice(&dev));
+  AuxEvents &e = ev[dev & 63];
+  if (!e.a) {
+    TRACS_CK(cudaEventCreateWithFlags(&e.a, cudaEventDisableTiming));
+    TRACS_CK(cudaEventCreateWithFlags(&e.b, cudaEventDisableTiming));
+  }
+  return e;
+}
+
 }  // namespace tracs
 #include "pairs.inl"
 namespace tracs {
 
 static void eval_finish_overlapped(const Ingested &g, const uint64_t *keys, uint64_t n_keys, uint32_t *d, uint32_t *u, uint64_t n,
                                    uint64_t L_total, const tracs_opts_t &o, TransLut *lut, HostEdges &out, cudaStream_t st);
+
+// Recombination filter (K4) of E sorted edges: filtered distances into filt32, and widened to the output type into filt64.
+static void recomb_filter(const Ingested &g, const uint64_t *keys, const uint32_t *dvals, uint64_t E, DevBuf<uint32_t> &filt32,
+                          DevBuf<uint64_t> &filt64, cudaStream_t st) {
+  tracs_stats_t &S = g_stats;
+  Timer T(st);
+  T.start();
+  filt32.alloc(E);
+  filt64.alloc(E);
+  DevBuf<uint64_t> offs(E + 1);
+  DevBuf<uint8_t> stmp;
+  size_t sb = 0;
+  TRACS_CK(cudaMemsetAsync(offs.p, 0, sizeof(uint64_t), st));
+  // the scan accumulates in the INPUT type: widen on the fly so offsets above 2^32 do not wrap
+  cub::TransformInputIterator<uint64_t, WidenU32, const uint32_t *> d_in64(dvals, WidenU32());
+  cub::DeviceScan::InclusiveSum(nullptr, sb, d_in64, offs.p + 1, (int64_t)E, st);
+  stmp.alloc(sb);
+  cub::DeviceScan::InclusiveSum(stmp.p, sb, d_in64, offs.p + 1, (int64_t)E, st);
+  uint64_t total = 0;
+  TRACS_CK(cudaMemcpyAsync(&total, offs.p + E, 8, cudaMemcpyDeviceToHost, st));
+  TRACS_CK(cudaStreamSynchronize(st));
+  const uint64_t LIMIT = 1ull << 29;  // SNP positions held at once (2 GB)
+  std::vector<uint64_t> cuts{0};
+  if (total > LIMIT) {
+    std::vector<uint64_t> h(E + 1);
+    TRACS_CK(cudaMemcpyAsync(h.data(), offs.p, (E + 1) * 8, cudaMemcpyDeviceToHost, st));
+    TRACS_CK(cudaStreamSynchronize(st));
+    uint64_t start = 0;
+    for (uint64_t e = 0; e < E; ++e) {
+      if (h[e + 1] - h[start] > LIMIT && e > start) {
+        cuts.push_back(e);
+        start = e;
+      }
+      if (h[e + 1] - h[e] > LIMIT) throw std::runtime_error("filter: a single pair has too many SNPs for the position scratch");
+    }
+    cuts.push_back(E);
+    // per-cut sizes
+    uint64_t mxn = 0;
+    for (size_t c = 0; c + 1 < cuts.size(); ++c) mxn = std::max(mxn, h[cuts[c + 1]] - h[cuts[c]]);
+    total = mxn;
+  } else {
+    cuts.push_back(E);
+  }
+  DevBuf<uint32_t> pos(std::max<uint64_t>(1, total));
+  const size_t nlg = 10000 + 16;
+  const auto lgh_keep = lgamma_table(nlg);
+  const std::vector<double> &lgh = *lgh_keep;
+  DevBuf<double> lg_f(nlg);
+  TRACS_CK(cudaMemcpyAsync(lg_f.p, lgh.data(), nlg * 8, cudaMemcpyHostToDevice, st));
+  for (size_t c = 0; c + 1 < cuts.size(); ++c) {
+    const uint64_t e0 = cuts[c], e1 = cuts[c + 1];
+    if (e1 == e0) continue;
+    uint64_t base = 0;
+    TRACS_CK(cudaMemcpyAsync(&base, offs.p + e0, 8, cudaMemcpyDeviceToHost, st));
+    TRACS_CK(cudaStreamSynchronize(st));
+    const unsigned grid = (unsigned)(((e1 - e0) * 32 + 255) / 256);
+    k_snp_positions<<<grid, 256, 0, st>>>(keys, e0, e1, g.planesT.p, g.Wp, g.site_idx.p, g.V, offs.p, base, pos.p);
+    k_filter_recomb<<<grid, 256, 0, st>>>(dvals, e0, e1, offs.p, base, pos.p, g.L, lg_f.p, filt32.p);
+    S.kernel_launches += 2;
+    TRACS_CK(cudaGetLastError());
+  }
+  k_widen<<<(unsigned)((E + 255) / 256), 256, 0, st>>>(filt32.p, E, filt64.p);
+  S.kernel_launches += 3;
+  S.ms_filter += T.stop();
+}
+
+// Sorted-edge tail of a thresholded sweep: the E edges in (c.keys, c.dv) are sorted and expanded into columns, given
+// their filtered distance, likelihood and compared sites, and appended to `out`. The columns leave for the host on the
+// auxiliary stream as soon as they exist, under the compared-sites kernel: (rows, cols, dist[, filt]) right away, the
+// likelihood columns after the transmission kernels (which therefore run BEFORE k_ncomp), the compared-sites column last
+// on the main stream. `keep_on_device`: also leave a packed copy of the columns on the device (tracs_edges_t.dev_packed).
+static void emit_sorted_edges(const Ingested &g, EdgeList &c, uint64_t E, int end_bit, const tracs_opts_t &o, TransLut *lut,
+                              bool keep_on_device, HostEdges &out, cudaStream_t st) {
+  tracs_stats_t &S = g_stats;
+  if (E == 0) return;
+  const bool want_n = o.want_ncomp != 0;
+  Timer T(st);
+  T.start();
+  size_t sort_bytes = 0;
+  cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, c.keys.p, c.keys2.p, c.dv.p, c.dv2.p, (int64_t)E, 0, end_bit, st);
+  DevBuf<uint8_t> sort_tmp(sort_bytes);
+  cub::DeviceRadixSort::SortPairs(sort_tmp.p, sort_bytes, c.keys.p, c.keys2.p, c.dv.p, c.dv2.p, (int64_t)E, 0, end_bit, st);
+  S.kernel_launches += 2 + (end_bit + 7) / 8;  // histogram + scan + one onesweep pass per 8 key bits
+  const uint64_t *keys = c.keys2.p;
+  const uint32_t *dv = c.dv2.p;
+  DevBuf<uint64_t> d_rows(E), d_cols(E), d_dist(E), d_nc;
+  k_expand<<<(unsigned)((E + 255) / 256), 256, 0, st>>>(keys, dv, E, d_rows.p, d_cols.p, d_dist.p);
+  S.kernel_launches++;
+  S.ms_sort += T.stop();
+
+  DevBuf<uint32_t> d_filt32;
+  DevBuf<uint64_t> d_filt64;
+  if (o.filter) recomb_filter(g, keys, dv, E, d_filt32, d_filt64, st);
+  const cudaStream_t aux = aux_stream();
+  const AuxEvents ev = aux_events();
+  const HostColumns dst = append_rows(out, E, want_n, o.filter != 0, lut != nullptr);
+  TRACS_CK(cudaEventRecord(ev.a, st));
+  TRACS_CK(cudaStreamWaitEvent(aux, ev.a, 0));
+  copy_columns(dst, {d_rows.p, d_cols.p, d_dist.p, nullptr, d_filt64.p, nullptr, nullptr, nullptr}, E, aux);
+  DevBuf<double> d_p0, d_eK, d_dt;
+  if (lut) {
+    T.start();
+    d_p0.alloc(E); d_eK.alloc(E); d_dt.alloc(E);
+    // with the filter on, the likelihood is fed the filtered distance (tracs/distance.py:182-192)
+    lut->apply(keys, o.filter ? d_filt32.p : dv, E, d_p0.p, d_eK.p, d_dt.p, st);
+    S.ms_trans += T.stop();
+    TRACS_CK(cudaEventRecord(ev.b, st));
+    TRACS_CK(cudaStreamWaitEvent(aux, ev.b, 0));
+    copy_columns(dst, {nullptr, nullptr, nullptr, nullptr, nullptr, d_p0.p, d_eK.p, d_dt.p}, E, aux);
+  }
+  if (want_n) {
+    T.start();
+    d_nc.alloc(E);
+    const uint32_t *order = nullptr;
+    DevBuf<uint32_t> rep, ok1, ok2, ov1, ov2;
+    DevBuf<uint8_t> otmp;
+    if (E >= 4096 && E < (1ull << 32)) {
+      rep.alloc(g.n); ok1.alloc(E); ok2.alloc(E); ov1.alloc(E); ov2.alloc(E);
+      k_rep_init<<<(unsigned)((g.n + 255) / 256), 256, 0, st>>>(rep.p, (uint32_t)g.n);
+      k_rep_min<<<(unsigned)((E + 255) / 256), 256, 0, st>>>(keys, E, rep.p);
+      k_rep_keys<<<(unsigned)((E + 255) / 256), 256, 0, st>>>(keys, E, rep.p, ok1.p, ov1.p);
+      size_t ob = 0;
+      cub::DeviceRadixSort::SortPairs(nullptr, ob, ok1.p, ok2.p, ov1.p, ov2.p, (int64_t)E, 0, end_bit - 32, st);
+      otmp.alloc(ob);
+      cub::DeviceRadixSort::SortPairs(otmp.p, ob, ok1.p, ok2.p, ov1.p, ov2.p, (int64_t)E, 0, end_bit - 32, st);
+      S.kernel_launches += 5 + (end_bit - 32 + 7) / 8;
+      order = ov2.p;
+    }
+    k_ncomp<<<(unsigned)((E * 32 + 255) / 256), 256, 0, st>>>(keys, E, g.nplane.p, g.npitch, g.nsum.p, g.spitch, g.ncount.p, g.L, order,
+                                                            d_nc.p);
+    S.kernel_launches++;
+    TRACS_CK(cudaGetLastError());
+    S.ms_ncomp += T.stop();
+  }
+  if (keep_on_device) {
+    void *dp = nullptr;
+    TRACS_CK(cudaMalloc(&dp, std::max<size_t>(32, 32 * E)));
+    out.dev_packed = dp;
+    out.dev_packed_bytes = 32 * E;
+    k_pack_edges<<<(unsigned)((E + 255) / 256), 256, 0, st>>>(keys, dv, want_n ? d_nc.p : nullptr, lut ? d_p0.p : nullptr,
+                                                             lut ? d_eK.p : nullptr, E, (uint8_t *)dp);
+    S.kernel_launches++;
+  }
+  T.start();
+  if (want_n) copy_columns(dst, {nullptr, nullptr, nullptr, d_nc.p, nullptr, nullptr, nullptr, nullptr}, E, st);
+  TRACS_CK(cudaStreamSynchronize(st));
+  TRACS_CK(cudaStreamSynchronize(aux));
+  S.ms_d2h += T.stop();
+  S.n_edges += E;
+}
+
+// Filter-and-refine over all of the plan's row-blocks (prefilter()), then every candidate is finished over the full
+// length: per component block (pairs.inl) with threshold, compared sites, likelihood and the copies to the host in one
+// go (eval_finish_overlapped), or -- filter=True, whose recombination filter needs the sorted edges -- per pair
+// (k_refine) followed by the sorted-edge tail. Returns false, with nothing appended, when the prefilter is not selective.
+static bool sweep_prefiltered(const Ingested &g, const TilePlan &plan, uint64_t pairs, const SweepArgs &a, bool tc_ok, int end_bit,
+                              const tracs_opts_t &o, TransLut *lut, HostEdges &out, cudaStream_t st) {
+  tracs_stats_t &S = g_stats;
+  EdgeList c(std::min(std::max<uint64_t>(1, pairs), CAND_CAP));
+  const Prefilter pf = prefilter(g, plan, pairs, a, tc_ok, c, st);
+  if (!pf.selective) return false;
+  const uint64_t n_cand = pf.n_cand;
+  if (n_cand == 0) return true;
+  Timer T(st);
+  if (!o.filter) {
+    // candidates in key order -> full-length d and |N u N| per candidate
+    T.start();
+    size_t kb = 0;
+    cub::DeviceRadixSort::SortKeys(nullptr, kb, c.keys.p, c.keys2.p, (int64_t)n_cand, 0, end_bit, st);
+    DevBuf<uint8_t> sort_tmp(kb);
+    cub::DeviceRadixSort::SortKeys(sort_tmp.p, kb, c.keys.p, c.keys2.p, (int64_t)n_cand, 0, end_bit, st);
+    S.kernel_launches += 2 + (end_bit + 7) / 8;
+    const bool want_n = o.want_ncomp != 0;
+    DevBuf<uint32_t> u_full(want_n ? n_cand : 1);
+    S.ms_refine += T.stop();
+    eval_finish_overlapped(g, c.keys2.p, n_cand, c.dv2.p, want_n ? u_full.p : nullptr, g.n, g.L, o, lut, out, st);
+    return true;
+  }
+  T.start();
+  c.reset(st);
+  k_refine<<<(unsigned)((n_cand * 32 + 255) / 256), 256, 0, st>>>(c.keys.p, c.dv.p, n_cand, g.planesT.p, g.Wp, pf.words, o.dist,
+                                                                 c.counter.p, c.keys2.p, c.dv2.p);
+  S.kernel_launches++;
+  TRACS_CK(cudaGetLastError());
+  S.ms_refine += T.stop();
+  const uint64_t E = c.count(st);
+  c.swap();  // survivors now in (keys, dv) like the plain sweep leaves them
+  emit_sorted_edges(g, c, E, end_bit, o, lut, o.keep_on_device != 0, out, st);
+  return true;
+}
+
+// Full-length sweep in bands whose pair count fits the edge buffer (a full-length sweep may emit every pair); each band's
+// edges go through the sorted-edge tail before the next band is swept. Ctrl-C is seen between bands.
+static void sweep_banded(const Ingested &g, const TilePlan &plan, SweepArgs a, bool tc_ok, int end_bit, const tracs_opts_t &o,
+                         TransLut *lut, HostEdges &out, cudaStream_t st) {
+  tracs_stats_t &S = g_stats;
+  const std::vector<Band> bands = make_bands(plan, BAND_PAIRS, BAND_TILES);
+  uint64_t cap = 1;
+  for (const Band &b : bands) cap = std::max(cap, b.pairs);
+  EdgeList c(cap);
+  c.output_to(a);
+  for (const Band &b : bands) {
+    check_interrupt();  // reference: PyErr_CheckSignals per row, src/pairsnp.hpp:385, 434-441
+    c.reset(st);
+    sweep_band(plan, b, a, tc_ok, g.has_n_var, false, st);
+    S.swept_wordpairs += b.pairs * std::max<uint64_t>(g.W, 1);  // algorithmic words (padding not counted)
+    const uint64_t E = c.count(st);
+    if (E > cap) throw std::runtime_error("internal error: edge buffer overflow");
+    emit_sorted_edges(g, c, E, end_bit, o, lut, o.keep_on_device && bands.size() == 1, out, st);
+  }
+}
 
 // Sweeps the device-resident ASCII matrix and appends edges (sorted) to `out`.
 void sweep_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint64_t pitch, const tracs_opts_t &o,
@@ -1731,340 +2094,44 @@ void sweep_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint64_t pitc
   const uint64_t j_start = o.j_start;
   if (n == 0 || i_end == 0 || j_start >= n) return;
   if (n >= (1ull << 31)) throw std::runtime_error("too many samples");
-
-  Timer T(st), Ttot(st);
+  Timer Ttot(st);
   Ttot.start();
-  const bool want_n = o.want_ncomp != 0;
+
+  // ---- ingest + plan ------------------------------------------------------------------------
   Ingested ing;
   ingest_device(dev_seqs, n, L, pitch, o.packed_input != 0, o.filter != 0, ing, st);
-  const uint64_t npitch = ing.npitch, spitch = ing.spitch, V = ing.V, W = ing.W;
-  const uint32_t Wp = ing.Wp, Npad = ing.Npad;
-  DevBuf<uint32_t> &nplane = ing.nplane, &ncount = ing.ncount, &site_idx = ing.site_idx;
-  DevBuf<uint8_t> &nsum = ing.nsum;
-  DevBuf<uint4> &planes = ing.planes, &planesT = ing.planesT;
-
-  // ---- tile lists ------------------------------------------------------------------------
   const int world = std::max(1, (int)o.shard_world), rank = std::max(0, (int)o.shard_rank);
-  const TilePlan plan = plan_tiles(n, i_end, j_start, Npad, rank, world);
-  const uint32_t n_cb = plan.n_cb, cb_min = plan.cb_min;
-  const std::vector<uint32_t> &my_rb = plan.my_rb;
-  // Units of work. A thresholded call first tries filter-and-refine over ALL owned row-blocks in one launch: the
-  // candidate list is bounded (CAND_CAP) because only a few per cent of the pairs may survive. Otherwise, or when the
-  // prefilter is not selective, the row-blocks are cut into bands whose pair count fits the edge buffer (a full-length
-  // sweep may emit every pair).
-  using Unit = Band;
-  const uint64_t CAP_MAX = BAND_PAIRS, CAND_CAP = 1ull << 26;
+  const TilePlan plan = plan_tiles(n, i_end, j_start, ing.Npad, rank, world);
   uint64_t total_pairs = 0, total_tiles = 0;
-  for (size_t k = 0; k < my_rb.size(); ++k) {
+  for (size_t k = 0; k < plan.my_rb.size(); ++k) {
     total_pairs += plan.rb_pairs[k];
-    total_tiles += n_cb - std::max(my_rb[k], cb_min);
+    total_tiles += plan.n_cb - std::max(plan.my_rb[k], plan.cb_min);
   }
   S.n_pairs += total_pairs;
-  auto make_units = [&](uint64_t limit, uint64_t tile_limit) { return make_bands(plan, limit, tile_limit); };
-  if (my_rb.empty()) {
+  if (plan.my_rb.empty()) {
     S.ms_total = Ttot.stop();
     return;
   }
-  const bool tc_ok = o.sweep_variant != 1 && !ing.partial_ambiguity;  // tensor cores unless forced off / inapplicable
-  bool prefilter_mode = o.sweep_variant == 0 && o.dist >= 0 && (uint64_t)o.dist < (uint64_t)PREFILTER_WORDS * 32 &&
-                        Wp >= 4 * PREFILTER_WORDS && total_tiles < (1ull << 31);
-
-  DevBuf<unsigned long long> counter(1);
-  DevBuf<uint32_t> d_rb(my_rb.size()), d_prefix(my_rb.size() + 1);
-  int end_bit = 32;
-  while ((1ull << (end_bit - 32)) < n) end_bit++;
+  const bool tc_ok = use_tensor_cores(o, ing);
+  // A thresholded call first tries filter-and-refine over ALL owned row-blocks in one launch per window (the candidate
+  // list is bounded: only a few per cent of the pairs may survive); otherwise, or when the prefilter is not selective,
+  // the banded full-length sweep (cost of the failed attempts: 92 / Wp).
+  const bool prefilter_mode = o.sweep_variant == 0 && o.dist >= 0 && (uint64_t)o.dist < (uint64_t)PREFILTER_WORDS * 32 &&
+                              ing.Wp >= 4 * PREFILTER_WORDS && total_tiles < BAND_TILES;
 
   // ---- fused transmission likelihood set-up (device table over (d, day difference)) ----------
   TransLut lut;
-  const bool fuse_trans = lut.setup(o, n, (uint64_t)std::min<int64_t>(std::max<int64_t>(o.dist, 0), (int64_t)Wp * 32) + 1, st);
+  const bool fuse_trans = lut.setup(o, n, (uint64_t)std::min<int64_t>(std::max<int64_t>(o.dist, 0), (int64_t)ing.Wp * 32) + 1, st);
   if (fuse_trans) out.has_trans = true;
 
-  for (int pass = 0; pass < 2; ++pass) {
-  const std::vector<Unit> units = prefilter_mode ? std::vector<Unit>{{0, my_rb.size(), total_pairs}} : make_units(CAP_MAX, 1ull << 31);
-  uint64_t cap = 1;
-  for (const Unit &u : units) cap = std::max(cap, u.pairs);
-  if (prefilter_mode) cap = std::min(cap, CAND_CAP);
-  DevBuf<uint64_t> keys(cap), keys2(cap);
-  DevBuf<uint32_t> dv(cap), dv2(cap);
-  size_t sort_tmp_bytes = 0;
-  cub::DeviceRadixSort::SortPairs(nullptr, sort_tmp_bytes, keys.p, keys2.p, dv.p, dv2.p, (int64_t)cap, 0, end_bit, st);
-  DevBuf<uint8_t> sort_tmp(sort_tmp_bytes);
-  bool fall_back = false;
-
-  for (size_t b = 0; b < units.size(); ++b) {
-    check_interrupt();  // Ctrl-C between bands (reference: PyErr_CheckSignals per row, src/pairsnp.hpp:385, 434-441)
-    std::vector<uint32_t> rbs(my_rb.begin() + units[b].first, my_rb.begin() + units[b].last);
-    std::vector<uint32_t> prefix(rbs.size() + 1, 0);
-    for (size_t k = 0; k < rbs.size(); ++k) prefix[k + 1] = prefix[k] + (n_cb - std::max(rbs[k], cb_min));
-    const uint32_t n_tiles = prefix.back();
-    TRACS_CK(cudaMemcpyAsync(d_rb.p, rbs.data(), rbs.size() * 4, cudaMemcpyHostToDevice, st));
-    TRACS_CK(cudaMemcpyAsync(d_prefix.p, prefix.data(), prefix.size() * 4, cudaMemcpyHostToDevice, st));
-    TRACS_CK(cudaMemsetAsync(counter.p, 0, sizeof(unsigned long long), st));
-    SweepArgs a;
-    a.planes = planes.p; a.Wp = Wp; a.Npad = Npad; a.n = (uint32_t)n; a.i_end = (uint32_t)i_end;
-    a.j_start = (uint32_t)j_start; a.dist = o.dist; a.rb_list = d_rb.p; a.tile_prefix = d_prefix.p;
-    a.n_rb = (uint32_t)rbs.size(); a.n_tiles = n_tiles; a.cb_min = cb_min; a.counter = counter.p;
-    a.keys = keys.p; a.dvals = dv.p; a.cap = cap; a.one = 1;
-    DevBuf<uint2> d_table(std::max<uint32_t>(1, n_tiles));
-    if (n_tiles) {
-      k_tile_table<<<(n_tiles + 255) / 256, 256, 0, st>>>(d_rb.p, d_prefix.p, a.n_rb, cb_min, n_tiles, d_table.p);
-      S.kernel_launches++;
-    }
-    a.tile_table = d_table.p;
-    auto read_counter = [&]() -> unsigned long long {
-      unsigned long long c = 0;
-      TRACS_CK(cudaMemcpyAsync(&c, counter.p, sizeof c, cudaMemcpyDeviceToHost, st));
-      TRACS_CK(cudaStreamSynchronize(st));
-      return c;
-    };
-    unsigned long long E = 0;
-    bool handled = false;
-    if (prefilter_mode) {
-      // Filter-and-refine: tile-sweep only the first words of every pair; d is monotone in the number of sites, so a
-      // pair whose partial distance already exceeds `dist` is decided. Windows of 4, 8, 16 and 64 words are tried in turn
-      // until <= 4 % of the pairs survive; those are finished per component / per pair (pairs.inl). If even the widest
-      // window is not selective the call falls back to banded full-length sweeps (cost of the failed attempts: 92 / Wp).
-      // Short windows run on the LOP3/POPC kernel (the tensor-core kernel pays its per-tile pipeline fill and its
-      // TMEM epilogue on every 128 x 128 tile: measured equal at 16 words, slower below), the 64-word one on the
-      // tensor cores when the masks allow it.
-      bool refined = false;
-      const uint32_t first = first_window(o.dist);
-      for (uint32_t pw = first; pw && !refined; pw = next_window(pw)) {
-        a.Wp = pw;
-        T.start();
-        launch_tile_sweep(a, tc_ok && pw >= tc_min_words(), st, ing.has_n_var);
-        S.ms_sweep += T.stop();
-        S.n_tiles += n_tiles;
-        S.swept_wordpairs += units[b].pairs * pw;
-        unsigned long long n_cand = read_counter();
-        TRACS_CK(cudaMemsetAsync(counter.p, 0, sizeof(unsigned long long), st));
-        if (n_cand && n_cand <= cap && n_cand * 25 <= units[b].pairs && pw < 16 && Wp > pw) {
-          // narrow window: trim the candidates over the next words, one thread each (k_cand_trim)
-          T.start();
-          const uint32_t extra = std::min<uint32_t>(Wp - pw, 32 - pw);
-          DevBuf<uint8_t> flags(n_cand);
-          DevBuf<uint64_t> n_sel(1);
-          k_cand_trim<<<(unsigned)((n_cand + 255) / 256), 256, 0, st>>>(keys.p, dv.p, n_cand, planesT.p, Wp, pw, extra, o.dist, flags.p);
-          size_t tb = 0;
-          cub::DeviceSelect::Flagged(nullptr, tb, keys.p, flags.p, keys2.p, n_sel.p, (int64_t)n_cand, st);
-          if (tb > sort_tmp_bytes) throw std::runtime_error("internal error: select scratch too small");
-          cub::DeviceSelect::Flagged(sort_tmp.p, tb, keys.p, flags.p, keys2.p, n_sel.p, (int64_t)n_cand, st);
-          cub::DeviceSelect::Flagged(sort_tmp.p, tb, dv.p, flags.p, dv2.p, n_sel.p, (int64_t)n_cand, st);
-          uint64_t kept = 0;
-          TRACS_CK(cudaMemcpyAsync(&kept, n_sel.p, 8, cudaMemcpyDeviceToHost, st));
-          TRACS_CK(cudaStreamSynchronize(st));
-          std::swap(keys.p, keys2.p);
-          std::swap(dv.p, dv2.p);
-          a.keys = keys.p; a.dvals = dv.p;
-          S.kernel_launches += 5;
-          S.ms_refine += T.stop();
-          n_cand = kept;
-        }
-        if (n_cand <= cap && n_cand * 25 <= units[b].pairs) {  // <= 4 % survive: per-pair refinement is cheaper than tiles
-          refined = true;
-          S.n_candidates += n_cand;
-          if (n_cand && !o.filter) {
-            // candidates in key order -> full-length d and |N u N| per candidate (component blocks, pairs.inl) ->
-            // threshold, compared sites, likelihood and the copy to the host in one go (the tail below is skipped)
-            T.start();
-            size_t kb = 0;
-            cub::DeviceRadixSort::SortKeys(nullptr, kb, keys.p, keys2.p, (int64_t)n_cand, 0, end_bit, st);
-            if (kb > sort_tmp_bytes) throw std::runtime_error("internal error: sort scratch too small");
-            cub::DeviceRadixSort::SortKeys(sort_tmp.p, kb, keys.p, keys2.p, (int64_t)n_cand, 0, end_bit, st);
-            S.kernel_launches += 2 + (end_bit + 7) / 8;
-            DevBuf<uint32_t> u_full(want_n ? n_cand : 1);
-            S.ms_refine += T.stop();
-            eval_finish_overlapped(ing, keys2.p, n_cand, dv2.p, want_n ? u_full.p : nullptr, n, L, o, fuse_trans ? &lut : nullptr, out, st);
-            handled = true;
-          } else if (n_cand) {
-            T.start();
-            k_refine<<<(unsigned)((n_cand * 32 + 255) / 256), 256, 0, st>>>(keys.p, dv.p, n_cand, planesT.p, Wp, pw, o.dist, counter.p,
-                                                                         keys2.p, dv2.p);
-            S.kernel_launches++;
-            TRACS_CK(cudaGetLastError());
-            S.ms_refine += T.stop();
-            E = read_counter();
-          }
-          std::swap(keys.p, keys2.p);  // survivors now in (keys, dv) like the plain sweep leaves them
-          std::swap(dv.p, dv2.p);
-        } else if (pw == PREFILTER_WORDS) {
-          S.n_candidates += n_cand;
-        }
-      }
-      if (!refined) {
-        fall_back = true;
-        break;
-      }
-      if (handled) continue;
-    } else {
-      // full-length sweep: the tensor-core kernel (2.0x the LOP3/POPC kernel at C2, profiles/r1_tc_ncu.md) whenever
-      // the masks allow its identity; variant 1 forces the LOP3/POPC kernel, variant 2 insists on tensor cores
-      if (o.sweep_variant == 2 && ing.partial_ambiguity)
-        throw std::runtime_error("tensor-core sweep requested but the alignment has 2-/3-base IUPAC codes at variable sites");
-      T.start();
-      launch_tile_sweep(a, tc_ok, st, ing.has_n_var);
-      S.ms_sweep += T.stop();
-      S.n_tiles += n_tiles;
-      S.swept_wordpairs += units[b].pairs * std::max<uint64_t>(W, 1);  // algorithmic words (padding not counted)
-      E = read_counter();
-    }
-    if (E > cap) throw std::runtime_error("internal error: edge buffer overflow");
-    if (E == 0) continue;
-
-    T.start();
-    cub::DeviceRadixSort::SortPairs(sort_tmp.p, sort_tmp_bytes, keys.p, keys2.p, dv.p, dv2.p, (int64_t)E, 0, end_bit, st);
-    S.kernel_launches += 2 + (end_bit + 7) / 8;  // histogram + scan + one onesweep pass per 8 key bits
-    DevBuf<uint64_t> d_rows(E), d_cols(E), d_dist(E), d_nc;
-    k_expand<<<(unsigned)((E + 255) / 256), 256, 0, st>>>(keys2.p, dv2.p, E, d_rows.p, d_cols.p, d_dist.p);
-    S.kernel_launches++;
-    S.ms_sort += T.stop();
-
-    DevBuf<uint32_t> d_filt32;
-    DevBuf<uint64_t> d_filt64;
-    if (o.filter) {
-      T.start();
-      d_filt32.alloc(E);
-      d_filt64.alloc(E);
-      DevBuf<uint64_t> offs(E + 1);
-      DevBuf<uint8_t> stmp;
-      size_t sb = 0;
-      TRACS_CK(cudaMemsetAsync(offs.p, 0, sizeof(uint64_t), st));
-      // the scan accumulates in the INPUT type: widen on the fly so offsets above 2^32 do not wrap
-      cub::TransformInputIterator<uint64_t, WidenU32, const uint32_t *> d_in64(dv2.p, WidenU32());
-      cub::DeviceScan::InclusiveSum(nullptr, sb, d_in64, offs.p + 1, (int64_t)E, st);
-      stmp.alloc(sb);
-      cub::DeviceScan::InclusiveSum(stmp.p, sb, d_in64, offs.p + 1, (int64_t)E, st);
-      uint64_t total = 0;
-      TRACS_CK(cudaMemcpyAsync(&total, offs.p + E, 8, cudaMemcpyDeviceToHost, st));
-      TRACS_CK(cudaStreamSynchronize(st));
-      const uint64_t LIMIT = 1ull << 29;  // SNP positions held at once (2 GB)
-      std::vector<uint64_t> cuts{0};
-      if (total > LIMIT) {
-        std::vector<uint64_t> h(E + 1);
-        TRACS_CK(cudaMemcpyAsync(h.data(), offs.p, (E + 1) * 8, cudaMemcpyDeviceToHost, st));
-        TRACS_CK(cudaStreamSynchronize(st));
-        uint64_t start = 0;
-        for (uint64_t e = 0; e < E; ++e) {
-          if (h[e + 1] - h[start] > LIMIT && e > start) {
-            cuts.push_back(e);
-            start = e;
-          }
-          if (h[e + 1] - h[e] > LIMIT) throw std::runtime_error("filter: a single pair has too many SNPs for the position scratch");
-        }
-        cuts.push_back(E);
-        // per-cut sizes
-        uint64_t mxn = 0;
-        for (size_t c = 0; c + 1 < cuts.size(); ++c) mxn = std::max(mxn, h[cuts[c + 1]] - h[cuts[c]]);
-        total = mxn;
-      } else {
-        cuts.push_back(E);
-      }
-      DevBuf<uint32_t> pos(std::max<uint64_t>(1, total));
-      const size_t nlg = 10000 + 16;
-      const auto lgh_keep = lgamma_table(nlg);
-      const std::vector<double> &lgh = *lgh_keep;
-      DevBuf<double> lg_f(nlg);
-      TRACS_CK(cudaMemcpyAsync(lg_f.p, lgh.data(), nlg * 8, cudaMemcpyHostToDevice, st));
-      for (size_t c = 0; c + 1 < cuts.size(); ++c) {
-        const uint64_t e0 = cuts[c], e1 = cuts[c + 1];
-        if (e1 == e0) continue;
-        uint64_t base = 0;
-        TRACS_CK(cudaMemcpyAsync(&base, offs.p + e0, 8, cudaMemcpyDeviceToHost, st));
-        TRACS_CK(cudaStreamSynchronize(st));
-        const unsigned g = (unsigned)(((e1 - e0) * 32 + 255) / 256);
-        k_snp_positions<<<g, 256, 0, st>>>(keys2.p, e0, e1, planesT.p, Wp, site_idx.p, V, offs.p, base, pos.p);
-        k_filter_recomb<<<g, 256, 0, st>>>(dv2.p, e0, e1, offs.p, base, pos.p, L, lg_f.p, d_filt32.p);
-        S.kernel_launches += 2;
-        TRACS_CK(cudaGetLastError());
-      }
-      k_widen<<<(unsigned)((E + 255) / 256), 256, 0, st>>>(d_filt32.p, E, d_filt64.p);
-      S.kernel_launches += 3;
-      S.ms_filter += T.stop();
-    }
-    // Edge columns leave for the host on a side stream as soon as they exist, under the compared-sites kernel:
-    // (rows, cols, dist[, filt]) right away, the likelihood columns after the transmission kernels (which therefore run
-    // BEFORE k_ncomp), the compared-sites column last on the main stream.
-    static thread_local cudaStream_t cs = nullptr;
-    static thread_local cudaEvent_t ev_cols = nullptr, ev_trans = nullptr;
-    static thread_local int cs_dev = -1;
-    int cur_dev = 0;
-    TRACS_CK(cudaGetDevice(&cur_dev));
-    if (!cs || cs_dev != cur_dev) {  // (a stream made for another device is left to the driver)
-      cs_dev = cur_dev;
-      TRACS_CK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
-      TRACS_CK(cudaEventCreateWithFlags(&ev_cols, cudaEventDisableTiming));
-      TRACS_CK(cudaEventCreateWithFlags(&ev_trans, cudaEventDisableTiming));
-    }
-    const size_t old = out.rows.size();
-    out.rows.resize(old + E); out.cols.resize(old + E); out.dist.resize(old + E);
-    if (want_n) out.ncomp.resize(old + E);
-    if (o.filter) out.filt.resize(old + E);
-    if (fuse_trans) { out.p0_log.resize(old + E); out.eK.resize(old + E); out.datediff.resize(old + E); }
-    TRACS_CK(cudaEventRecord(ev_cols, st));
-    TRACS_CK(cudaStreamWaitEvent(cs, ev_cols, 0));
-    if (o.filter) TRACS_CK(cudaMemcpyAsync(out.filt.data() + old, d_filt64.p, E * 8, cudaMemcpyDeviceToHost, cs));
-    TRACS_CK(cudaMemcpyAsync(out.rows.data() + old, d_rows.p, E * 8, cudaMemcpyDeviceToHost, cs));
-    TRACS_CK(cudaMemcpyAsync(out.cols.data() + old, d_cols.p, E * 8, cudaMemcpyDeviceToHost, cs));
-    TRACS_CK(cudaMemcpyAsync(out.dist.data() + old, d_dist.p, E * 8, cudaMemcpyDeviceToHost, cs));
-    DevBuf<double> d_p0, d_eK, d_dt;
-    if (fuse_trans) {
-      T.start();
-      d_p0.alloc(E); d_eK.alloc(E); d_dt.alloc(E);
-      // with the filter on, the likelihood is fed the filtered distance (tracs/distance.py:182-192)
-      lut.apply(keys2.p, o.filter ? d_filt32.p : dv2.p, E, d_p0.p, d_eK.p, d_dt.p, st);
-      S.ms_trans += T.stop();
-      TRACS_CK(cudaEventRecord(ev_trans, st));
-      TRACS_CK(cudaStreamWaitEvent(cs, ev_trans, 0));
-      TRACS_CK(cudaMemcpyAsync(out.p0_log.data() + old, d_p0.p, E * 8, cudaMemcpyDeviceToHost, cs));
-      TRACS_CK(cudaMemcpyAsync(out.eK.data() + old, d_eK.p, E * 8, cudaMemcpyDeviceToHost, cs));
-      TRACS_CK(cudaMemcpyAsync(out.datediff.data() + old, d_dt.p, E * 8, cudaMemcpyDeviceToHost, cs));
-      S.d2h_bytes += E * 24;
-    }
-    if (want_n) {
-      T.start();
-      d_nc.alloc(E);
-      const uint32_t *order = nullptr;
-      DevBuf<uint32_t> rep, ok1, ok2, ov1, ov2;
-      DevBuf<uint8_t> otmp;
-      if (E >= 4096 && E < (1ull << 32)) {
-        rep.alloc(n); ok1.alloc(E); ok2.alloc(E); ov1.alloc(E); ov2.alloc(E);
-        k_rep_init<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(rep.p, (uint32_t)n);
-        k_rep_min<<<(unsigned)((E + 255) / 256), 256, 0, st>>>(keys2.p, E, rep.p);
-        k_rep_keys<<<(unsigned)((E + 255) / 256), 256, 0, st>>>(keys2.p, E, rep.p, ok1.p, ov1.p);
-        size_t ob = 0;
-        cub::DeviceRadixSort::SortPairs(nullptr, ob, ok1.p, ok2.p, ov1.p, ov2.p, (int64_t)E, 0, end_bit - 32, st);
-        otmp.alloc(ob);
-        cub::DeviceRadixSort::SortPairs(otmp.p, ob, ok1.p, ok2.p, ov1.p, ov2.p, (int64_t)E, 0, end_bit - 32, st);
-        S.kernel_launches += 5 + (end_bit - 32 + 7) / 8;
-        order = ov2.p;
-      }
-      k_ncomp<<<(unsigned)((E * 32 + 255) / 256), 256, 0, st>>>(keys2.p, E, nplane.p, npitch, nsum.p, spitch, ncount.p, L, order,
-                                                              d_nc.p);
-      S.kernel_launches++;
-      TRACS_CK(cudaGetLastError());
-      S.ms_ncomp += T.stop();
-    }
-    if (o.keep_on_device && units.size() == 1) {
-      void *dp = nullptr;
-      TRACS_CK(cudaMalloc(&dp, std::max<size_t>(32, 32 * E)));
-      out.dev_packed = dp;
-      out.dev_packed_bytes = 32 * E;
-      k_pack_edges<<<(unsigned)((E + 255) / 256), 256, 0, st>>>(keys2.p, dv2.p, want_n ? d_nc.p : nullptr,
-                                                               fuse_trans ? d_p0.p : nullptr, fuse_trans ? d_eK.p : nullptr, E,
-                                                               (uint8_t *)dp);
-      S.kernel_launches++;
-    }
-    T.start();
-    if (want_n) TRACS_CK(cudaMemcpyAsync(out.ncomp.data() + old, d_nc.p, E * 8, cudaMemcpyDeviceToHost, st));
-    TRACS_CK(cudaStreamSynchronize(st));
-    TRACS_CK(cudaStreamSynchronize(cs));
-    S.ms_d2h += T.stop();
-    S.d2h_bytes += E * 8 * (want_n ? 4 : 3);
-    S.n_edges += E;
+  const int end_bit = key_end_bit(n);
+  const SweepArgs a = sweep_args(ing, i_end, j_start, o.dist);
+  bool done = false;
+  if (prefilter_mode) {
+    check_interrupt();
+    done = sweep_prefiltered(ing, plan, total_pairs, a, tc_ok, end_bit, o, fuse_trans ? &lut : nullptr, out, st);
   }
-  if (!fall_back) break;
-  prefilter_mode = false;  // second pass: banded full-length sweeps
-  }
+  if (!done) sweep_banded(ing, plan, a, tc_ok, end_bit, o, fuse_trans ? &lut : nullptr, out, st);
   S.ms_total = Ttot.stop();
 }
 
@@ -2081,40 +2148,18 @@ void distance_matrix_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uin
   if (n == 0 || i_end == 0 || j_start >= n) return;
   if (n >= (1ull << 31)) throw std::runtime_error("too many samples");
   const bool square = j_start == 0;
-  Timer T(st), Ttot(st);
+  Timer Ttot(st);
   Ttot.start();
   Ingested ing;
   ingest_device(dev_seqs, n, L, pitch, o.packed_input != 0, false, ing, st);
-  if (o.sweep_variant == 2 && ing.partial_ambiguity)
-    throw std::runtime_error("tensor-core sweep requested but the alignment has 2-/3-base IUPAC codes at variable sites");
-  const bool use_tc = o.sweep_variant != 1 && !ing.partial_ambiguity;
+  const bool use_tc = use_tensor_cores(o, ing);
   const TilePlan plan = plan_tiles(n, i_end, j_start, ing.Npad, 0, 1);
+  SweepArgs a = sweep_args(ing, i_end, j_start, INT32_MAX);
+  a.dense = out; a.dense_ld = ld; a.dense_col0 = (uint32_t)j_start; a.dense_mirror = square ? 1u : 0u;
   // bands as on the sparse path: one launch each, Ctrl-C is seen between them
-  const std::vector<Band> bands = make_bands(plan, BAND_PAIRS, 1ull << 31);
-  DevBuf<uint32_t> d_rb(std::max<size_t>(1, plan.my_rb.size())), d_prefix(plan.my_rb.size() + 1);
-  for (const Band &b : bands) {
+  for (const Band &b : make_bands(plan, BAND_PAIRS, BAND_TILES)) {
     check_interrupt();
-    std::vector<uint32_t> rbs(plan.my_rb.begin() + b.first, plan.my_rb.begin() + b.last);
-    std::vector<uint32_t> prefix(rbs.size() + 1, 0);
-    for (size_t k = 0; k < rbs.size(); ++k) prefix[k + 1] = prefix[k] + (plan.n_cb - std::max(rbs[k], plan.cb_min));
-    const uint32_t n_tiles = prefix.back();
-    TRACS_CK(cudaMemcpyAsync(d_rb.p, rbs.data(), rbs.size() * 4, cudaMemcpyHostToDevice, st));
-    TRACS_CK(cudaMemcpyAsync(d_prefix.p, prefix.data(), prefix.size() * 4, cudaMemcpyHostToDevice, st));
-    SweepArgs a;
-    a.planes = ing.planes.p; a.Wp = ing.Wp; a.Npad = ing.Npad; a.n = (uint32_t)n; a.i_end = (uint32_t)i_end;
-    a.j_start = (uint32_t)j_start; a.dist = INT32_MAX; a.rb_list = d_rb.p; a.tile_prefix = d_prefix.p;
-    a.n_rb = (uint32_t)rbs.size(); a.n_tiles = n_tiles; a.cb_min = plan.cb_min; a.one = 1; a.tc_ncnt = nullptr;
-    a.dense = out; a.dense_ld = ld; a.dense_col0 = (uint32_t)j_start; a.dense_mirror = square ? 1u : 0u;
-    DevBuf<uint2> d_table(std::max<uint32_t>(1, n_tiles));
-    if (n_tiles) {
-      k_tile_table<<<(n_tiles + 255) / 256, 256, 0, st>>>(d_rb.p, d_prefix.p, a.n_rb, plan.cb_min, n_tiles, d_table.p);
-      S.kernel_launches++;
-    }
-    a.tile_table = d_table.p;
-    T.start();
-    launch_tile_sweep(a, use_tc, st, ing.has_n_var, true);
-    S.ms_sweep += T.stop();
-    S.n_tiles += n_tiles;
+    sweep_band(plan, b, a, use_tc, ing.has_n_var, true, st);
     S.n_pairs += b.pairs;
     S.swept_wordpairs += b.pairs * std::max<uint64_t>(ing.W, 1);
   }
