@@ -154,6 +154,43 @@ int tracs_distance_matrix_host(const uint8_t *seqs, size_t n, size_t L, size_t p
 int tracs_write_distance_matrix(const char *path, const int32_t *m, size_t rows, size_t cols, size_t ld,
                                 const char *const *row_names, const char *const *col_names, char sep);
 
+/* ---- resident sample database (query x db without re-ingesting the database) ----------------------------------------
+ * The two-file mode of pairsnp (rows = new samples, cols = a database) for callers that place batch after batch of new
+ * samples against the same collection: the database is ingested once (N-plane, variable sites, bit-planes) and stays on the
+ * device; each query pays for its own rows and its own pairs. For a database db (n_db samples, L sites) and a query batch
+ * q (nq samples, the same L):
+ *   tracs_db_query_*(db, q, opts)  returns exactly what  tracs_pairsnp_host([q; db], opts with i_end = j_start = nq)
+ * returns: every column, the same (row, col) order, two-file indices (rows in [0, nq), cols in [nq, nq + n_db)).
+ * opts as on the two-file call: dist, want_ncomp, sweep_variant, packed_input (of the query rows), want_trans / days (nq + n_db
+ * days, queries first) / lamb / beta / threshold_Ek. Refused before any device call, naming the field: filter, keep_on_device,
+ * shard_world > 1, i_end or j_start set, a bad pitch, a NULL or closed handle. nq = 0 returns no edges.
+ * A query whose bit-planes do not fit in device memory fails with their size in GB; the handle stays usable.
+ * tracs_last_stats after a query describes the query's own work (n_pairs = nq * n_db).
+ *
+ * open: opts may be NULL; only opts->packed_input is read (ASCII rows, or 4-bit rows as tracs_pairsnp_packed).
+ *   _host copies the rows into device memory the library owns (streamed like tracs_pairsnp_host).
+ *   _device with 4-bit rows BORROWS dev_seqs until tracs_db_close: unlike every other entry point, the buffer must stay allocated
+ *   and unchanged while the handle is open (the library only reads it; a second copy of a 100 GB database would not fit).
+ *   _device with ASCII rows encodes them once into 4-bit rows the library owns (half their size); dev_seqs is not kept.
+ * The handle belongs to the device that was current at open; a query while another device is current fails. Closing a handle
+ * twice, or passing one that was never opened, fails without touching memory. */
+typedef struct tracs_db_info {
+  uint64_t n;                /* database samples                                                   */
+  uint64_t L;                /* sites                                                              */
+  uint64_t n_variable_sites; /* variable sites of the database alone                               */
+  int32_t device;            /* the device the handle belongs to                                   */
+  int32_t reserved0;
+  uint64_t bytes_held;       /* device bytes the handle holds (borrowed rows not counted)          */
+  uint64_t query_rows;       /* query rows swept at once; larger batches go through in chunks       */
+  uint64_t new_sites;        /* sites variable in [q; db] but not in db, for the last query batch  */
+} tracs_db_info_t;
+int tracs_db_open_host(const uint8_t *seqs, size_t n, size_t L, size_t pitch, const tracs_opts_t *opts, void **db);
+int tracs_db_open_device(const uint8_t *dev_seqs, size_t n, size_t L, size_t pitch, const tracs_opts_t *opts, void **db);
+int tracs_db_query_host(void *db, const uint8_t *seqs, size_t nq, size_t pitch, const tracs_opts_t *opts, tracs_edges_t *out);
+int tracs_db_query_device(void *db, const uint8_t *dev_seqs, size_t nq, size_t pitch, const tracs_opts_t *opts, tracs_edges_t *out);
+int tracs_db_info(void *db, tracs_db_info_t *out);
+int tracs_db_close(void *db);
+
 /* ASCII rows -> packed rows on the device (what the host-streaming path runs per chunk): dev_ascii[rows][pitch]
  * (pitch % 32 == 0, >= L rounded up to 32) -> dev_nib[rows][pitch_bytes]. Sites >= L become 1111. */
 int tracs_encode_packed(const uint8_t *dev_ascii, size_t rows, size_t L, size_t pitch, uint8_t *dev_nib, size_t pitch_bytes);

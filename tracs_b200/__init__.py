@@ -8,7 +8,8 @@ import sys
 
 from .api import (pairsnp, trans_dist, lprob_k_given_N, calculate_posteriors, pairsnp_matrix, pairsnp_device, pairsnp_packed,
                   pairsnp_packed_host, pack_nibbles, distance_matrix, distance_matrix_device, write_distance_matrix,
-                  min_over_refs, synth_device, int_peak, tc_peak, tc_peak_sustained, last_stats, read_fasta, shard_rowblocks, connected_components, INT32_MAX)
+                  min_over_refs, synth_device, int_peak, tc_peak, tc_peak_sustained, last_stats, read_fasta, shard_rowblocks, connected_components, Database,
+                  INT32_MAX)
 
 DROPIN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "dropin")
 

@@ -39,6 +39,14 @@ class Opts(C.Structure):
                 ("packed_input", C.c_int32), ("reserved0", C.c_int32)]
 
 
+class DbInfo(C.Structure):
+    _fields_ = [("n", C.c_uint64), ("L", C.c_uint64), ("n_variable_sites", C.c_uint64), ("device", C.c_int32), ("reserved0", C.c_int32),
+                ("bytes_held", C.c_uint64), ("query_rows", C.c_uint64), ("new_sites", C.c_uint64)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
 class Synth(C.Structure):
     _fields_ = [("n", C.c_uint64), ("L", C.c_uint64), ("pitch", C.c_uint64), ("seed", C.c_uint64), ("p_var", C.c_double),
                 ("n_clusters", C.c_uint32), ("mu", C.c_double), ("p_N", C.c_double), ("p_amb", C.c_double),
@@ -55,7 +63,8 @@ SYMBOLS = ["tracs_pairsnp", "tracs_pairsnp_host", "tracs_pairsnp_device", "tracs
            "tracs_site_shard_open", "tracs_site_shard_partials", "tracs_site_shard_close", "tracs_connected_components",
            "tracs_write_distance_csv", "tracs_float_repr", "tracs_pairsnp_packed", "tracs_encode_packed", "tracs_site_shard_finish", "tracs_tc_peak", "tracs_tc_peak_sustained", "tracs_site_shard_select", "tracs_site_shard_emit",
            "tracs_host_register", "tracs_host_unregister", "tracs_distance_matrix_device", "tracs_distance_matrix_host",
-           "tracs_write_distance_matrix"]
+           "tracs_write_distance_matrix", "tracs_db_open_host", "tracs_db_open_device", "tracs_db_query_host", "tracs_db_query_device",
+           "tracs_db_info", "tracs_db_close"]
 
 _lib = None
 
@@ -115,6 +124,12 @@ def lib():
         L.tracs_distance_matrix_host.argtypes = [C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.POINTER(Opts), C.c_void_p, C.c_size_t]
         L.tracs_write_distance_matrix.argtypes = [C.c_char_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.POINTER(C.c_char_p),
                                                   C.POINTER(C.c_char_p), C.c_char]
+        L.tracs_db_open_host.argtypes = [C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.POINTER(Opts), C.POINTER(C.c_void_p)]
+        L.tracs_db_open_device.argtypes = [C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.POINTER(Opts), C.POINTER(C.c_void_p)]
+        L.tracs_db_query_host.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.POINTER(Opts), C.POINTER(Edges)]
+        L.tracs_db_query_device.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.POINTER(Opts), C.POINTER(Edges)]
+        L.tracs_db_info.argtypes = [C.c_void_p, C.POINTER(DbInfo)]
+        L.tracs_db_close.argtypes = [C.c_void_p]
         _lib = L
     return _lib
 

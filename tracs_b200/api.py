@@ -218,6 +218,113 @@ def write_distance_matrix(path, m, row_names, col_names, sep="\t", n_threads=Non
                 os.environ["TRACS_WRITE_THREADS"] = old
 
 
+class Database:
+    """A sample collection ingested once and kept on the GPU, against which batches of new samples are placed: the two-file
+    (query x db) mode of pairsnp without ingesting the database again on every call.
+
+    query(q) returns exactly what pairsnp_matrix(concatenate([q, db]), i_end=nq, j_start=nq) returns: the same columns in the
+    same order, rows = query index in [0, nq), cols = nq + database index. `days` (for the transmission likelihood) covers
+    the queries first, then the database. Not supported: the recombination filter, query x query pairs.
+
+    Database(seqs) copies a host matrix (ASCII uint8[n][L], or pack_nibbles rows with packed=True and L) into device memory
+    the handle owns. Use it as a context manager, or close() it, to release that memory."""
+
+    def __init__(self, seqs=None, packed=False, L=None, _handle=None, _keep=None):
+        self._h = None
+        self._keep = _keep
+        self.names = None
+        if _handle is not None:
+            self._h = _handle
+        else:
+            seqs = np.ascontiguousarray(seqs, dtype=np.uint8)
+            if seqs.ndim != 2:
+                raise ValueError("seqs must be a 2-D uint8 matrix")
+            n, width = seqs.shape
+            if packed and L is None:
+                raise ValueError("L (sites) is required with packed=True")
+            L = width if L is None else int(L)
+            o, _ = make_opts(packed=packed)
+            h = C.c_void_p()
+            _lib.check(_lib.lib().tracs_db_open_host(seqs.ctypes.data, n, L, width, C.byref(o), C.byref(h)))
+            self._h = h.value
+        self.n, self.L = self.info()["n"], self.info()["L"]
+
+    @classmethod
+    def from_device(cls, ptr, n, L, pitch, packed=False):
+        """A database over a DEVICE buffer (raw pointer as int; ASCII rows, or 4-bit rows with packed=True). A 4-bit buffer is
+        BORROWED, not copied: it must stay allocated and unchanged until close(); the library never writes to it. ASCII rows are
+        encoded once into 4-bit rows the handle owns, and the buffer is not kept."""
+        o, _ = make_opts(packed=packed)
+        h = C.c_void_p()
+        _lib.check(_lib.lib().tracs_db_open_device(C.c_void_p(ptr), int(n), int(L), int(pitch), C.byref(o), C.byref(h)))
+        return cls(_handle=h.value)
+
+    @classmethod
+    def from_fasta(cls, path, n_threads=1):
+        """A database from a FASTA(.gz) file (read into host memory first with read_fasta); keeps the sample names."""
+        seqs, names = read_fasta(path, n_threads)
+        db = cls(seqs)
+        db.names = names
+        return db
+
+    def _opts(self, dist, days, want_ncomp, full_sweep, packed, nq):
+        if days is not None and len(days) != nq + self.n:
+            raise ValueError("days must hold nq + n_db = %d values (queries first, then the database)" % (nq + self.n))
+        return make_opts(dist=dist, days=days, want_ncomp=want_ncomp, full_sweep=full_sweep, packed=packed)
+
+    def query(self, seqs, dist=INT32_MAX, days=None, want_ncomp=True, full_sweep=False, packed=False, L=None):
+        """Edges between the HOST query rows (ASCII uint8[nq][L], or pack_nibbles rows with packed=True) and the database,
+        as the dict of pairsnp_matrix."""
+        seqs = np.ascontiguousarray(seqs, dtype=np.uint8)
+        if seqs.ndim != 2:
+            raise ValueError("seqs must be a 2-D uint8 matrix")
+        nq, width = seqs.shape
+        L = (width if not packed else self.L) if L is None else int(L)
+        if L != self.L:
+            raise ValueError("query L (%d sites) differs from the database's L (%d sites)" % (L, self.L))
+        o, keep = self._opts(dist, days, want_ncomp, full_sweep, packed, nq)
+        e = Edges()
+        _lib.check(_lib.lib().tracs_db_query_host(C.c_void_p(self._handle()), seqs.ctypes.data, nq, width, C.byref(o), C.byref(e)))
+        return _lib.take_edges(e, names=False)
+
+    def query_device(self, ptr, nq, pitch, dist=INT32_MAX, days=None, want_ncomp=True, full_sweep=False, packed=False):
+        """query() on DEVICE query rows (raw pointer as int; ASCII rows, or 4-bit rows with packed=True) of the database's L."""
+        o, keep = self._opts(dist, days, want_ncomp, full_sweep, packed, int(nq))
+        e = Edges()
+        _lib.check(_lib.lib().tracs_db_query_device(C.c_void_p(self._handle()), C.c_void_p(ptr), int(nq), int(pitch), C.byref(o), C.byref(e)))
+        return _lib.take_edges(e, names=False)
+
+    def info(self):
+        """n, L, n_variable_sites (of the database), device, bytes_held, query_rows (swept at once) and new_sites (sites
+        that the last query batch made variable)."""
+        i = _lib.DbInfo()
+        _lib.check(_lib.lib().tracs_db_info(C.c_void_p(self._handle()), C.byref(i)))
+        return i.as_dict()
+
+    def _handle(self):
+        if self._h is None:
+            raise RuntimeError("database: the handle is closed")
+        return self._h
+
+    def close(self):
+        """Releases the device memory the handle holds (a borrowed buffer stays the caller's). Closing twice is harmless."""
+        if self._h is not None:
+            h, self._h = self._h, None
+            _lib.check(_lib.lib().tracs_db_close(C.c_void_p(h)))
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 def min_over_refs(a, b, val):
     """Min-over-references combine (SURVEY A.6): unordered (a,b) -> min(val). Sorted by (lo, hi)."""
     a = np.ascontiguousarray(a, dtype=np.uint64)

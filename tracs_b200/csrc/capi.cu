@@ -9,6 +9,7 @@
 #include <functional>
 #include <numeric>
 #include <map>
+#include <set>
 #include <mutex>
 #include <stdexcept>
 #include <string>
@@ -485,9 +486,11 @@ static void h2d_rows(uint8_t *dev, size_t dpitch, const uint8_t *src, size_t spi
 // c + 1 (copy stream) overlaps the ASCII -> nibble encode of chunk c (compute stream), and only two ASCII chunks are
 // ever resident, so an alignment whose ASCII form exceeds the device (100 000 x 2 Mb = 200 GB) still goes through.
 // A host matrix that is already packed is copied straight into place.
+static size_t packed_pitch(size_t L) { return std::max<size_t>(16, (L + 31) / 32 * 16); }
+
 static void stream_host_to_packed(const uint8_t *seqs, size_t n, size_t L, size_t hpitch, bool host_is_packed, DevBuf<uint8_t> &nib,
                                   size_t &pitch4, cudaStream_t st) {
-  pitch4 = std::max<size_t>(16, (L + 31) / 32 * 16);
+  pitch4 = packed_pitch(L);
   nib.alloc(n * pitch4);
   if (n == 0 || L == 0) return;
   if (host_is_packed) {
@@ -707,6 +710,19 @@ namespace tracs {
 struct DenseShape {
   uint64_t rows = 0, cols = 0;
 };
+// Pitch of an input matrix of n rows: host rows hold L ASCII bytes or (L + 1) / 2 packed bytes; device rows follow the
+// ingest's alignment rules. Host code only.
+static void check_pitch(const char *pre, size_t pitch, size_t L, bool packed, bool host_input, size_t n) {
+  bool pitch_ok;
+  if (host_input) pitch_ok = packed ? pitch >= (L + 1) / 2 : pitch >= L;
+  else if (packed) pitch_ok = pitch % 16 == 0 && pitch * 2 >= std::max<size_t>(32, (L + 31) / 32 * 32);
+  else pitch_ok = pitch % 32 == 0 && pitch >= (L + 31) / 32 * 32;
+  if (!pitch_ok && n > 0)
+    throw std::runtime_error(std::string(pre) + "pitch (" + std::to_string(pitch) + ") " +
+                             (host_input ? (packed ? "must hold (L + 1) / 2 bytes" : "must be >= L")
+                                         : (packed ? "must be a multiple of 16 bytes and hold L rounded up to 32 sites"
+                                                   : "must be a multiple of 32 and >= L rounded up to 32")));
+}
 // Argument check of the dense entry points. Host code only (no device call), so it runs before require_device().
 static DenseShape dense_check(const tracs_opts_t *opts, size_t n, size_t L, size_t pitch, size_t ld, const void *out, bool host_input) {
   const tracs_opts_t o = normalise(opts, n);
@@ -733,15 +749,7 @@ static DenseShape dense_check(const tracs_opts_t *opts, size_t n, size_t L, size
   if (ld < sh.cols) throw std::runtime_error(std::string(pre) + "ld (" + std::to_string(ld) + ") is smaller than the column count (" + std::to_string(sh.cols) + ")");
   if (!out && sh.rows && sh.cols) throw std::runtime_error(std::string(pre) + "out is NULL");
   const bool packed = o.packed_input != 0;
-  bool pitch_ok;
-  if (host_input) pitch_ok = packed ? pitch >= (L + 1) / 2 : pitch >= L;
-  else if (packed) pitch_ok = pitch % 16 == 0 && pitch * 2 >= std::max<size_t>(32, (L + 31) / 32 * 32);
-  else pitch_ok = pitch % 32 == 0 && pitch >= (L + 31) / 32 * 32;
-  if (!pitch_ok && n > 0)
-    throw std::runtime_error(std::string(pre) + "pitch (" + std::to_string(pitch) + ") " +
-                             (host_input ? (packed ? "must hold (L + 1) / 2 bytes" : "must be >= L")
-                                         : (packed ? "must be a multiple of 16 bytes and hold L rounded up to 32 sites"
-                                                   : "must be a multiple of 32 and >= L rounded up to 32")));
+  check_pitch(pre, pitch, L, packed, host_input, n);
   return sh;
 }
 
@@ -815,6 +823,161 @@ int tracs_distance_matrix_host(const uint8_t *seqs, size_t n, size_t L, size_t p
       g_stats.ms_total += g_stats.ms_d2h;
       g_stats.d2h_bytes += m_bytes;
     });
+  });
+}
+
+}  // extern "C"
+
+// ---- resident sample database (tracs_db_*) ----------------------------------------------------------------------
+namespace tracs {
+namespace {
+std::mutex g_db_mu;
+std::set<ResidentDb *> g_db_live;  // handles between open and close: anything else is refused, never dereferenced
+}  // namespace
+
+static ResidentDb *db_lookup(void *h) {
+  std::lock_guard<std::mutex> g(g_db_mu);
+  auto it = g_db_live.find((ResidentDb *)h);
+  if (!h || it == g_db_live.end()) throw std::runtime_error("database: the handle is NULL, closed, or was never opened");
+  return *it;
+}
+
+static void db_register(ResidentDb *db) {
+  std::lock_guard<std::mutex> g(g_db_mu);
+  g_db_live.insert(db);
+}
+
+// Argument check of tracs_db_query_*. Host code only, so it runs before require_device().
+static tracs_opts_t db_query_check(void *h, size_t nq, size_t pitch, const tracs_opts_t *opts, const tracs_edges_t *out, bool host_input,
+                                   ResidentDb *&db, uint64_t &L) {
+  const char *pre = "database query: ";
+  if (!out) throw std::runtime_error(std::string(pre) + "out is NULL");
+  tracs_opts_t o;
+  if (opts) o = *opts; else { memset(&o, 0, sizeof o); o.dist = INT32_MAX; o.want_ncomp = 1; }
+  if (o.filter) throw std::runtime_error(std::string(pre) + "opts->filter (recombination filter) is not supported against a database");
+  if (o.keep_on_device) throw std::runtime_error(std::string(pre) + "opts->keep_on_device is not supported against a database");
+  if (o.shard_world > 1) throw std::runtime_error(std::string(pre) + "opts->shard_world > 1: a database is swept on one GPU");
+  if (o.i_end || o.j_start)
+    throw std::runtime_error(std::string(pre) + "opts->i_end / opts->j_start must be 0: rows are the queries, cols the database");
+  if (o.sweep_variant < 0 || o.sweep_variant > 2) throw std::runtime_error(std::string(pre) + "opts->sweep_variant must be 0, 1 or 2");
+  if (nq >= (1ull << 31)) throw std::runtime_error(std::string(pre) + "nq: too many samples");
+  db = db_lookup(h);
+  tracs_db_info_t info;
+  db_info(*db, info);
+  L = info.L;
+  check_pitch(pre, pitch, L, o.packed_input != 0, host_input, nq);
+  o.shard_world = 1;
+  o.shard_rank = 0;
+  return o;
+}
+
+static void db_open_check(size_t n, size_t L, size_t pitch, const tracs_opts_t *opts, void **db, bool host_input) {
+  const char *pre = "database open: ";
+  if (!db) throw std::runtime_error(std::string(pre) + "db (the handle's address) is NULL");
+  *db = nullptr;
+  if (n == 0) throw std::runtime_error(std::string(pre) + "n must be at least 1");
+  if (n >= (1ull << 31) - 1024) throw std::runtime_error(std::string(pre) + "n: too many samples");
+  check_pitch(pre, pitch, L, opts && opts->packed_input, host_input, n);
+}
+}  // namespace tracs
+
+extern "C" {
+
+int tracs_db_open_host(const uint8_t *seqs, size_t n, size_t L, size_t pitch, const tracs_opts_t *opts, void **db) {
+  memset(&g_stats, 0, sizeof g_stats);
+  return guarded([&] {
+    db_open_check(n, L, pitch, opts, db, true);
+    require_device();
+    InterruptScope sigint;
+    DevBuf<uint8_t> nib;
+    size_t pitch4 = 0;
+    stream_host_to_packed(seqs, n, L, pitch, opts && opts->packed_input, nib, pitch4, 0);
+    const uint8_t *rows = nib.p;
+    ResidentDb *h = db_open(rows, n, L, pitch4, &nib, 0);
+    db_register(h);
+    *db = h;
+  });
+}
+
+int tracs_db_open_device(const uint8_t *dev_seqs, size_t n, size_t L, size_t pitch, const tracs_opts_t *opts, void **db) {
+  memset(&g_stats, 0, sizeof g_stats);
+  return guarded([&] {
+    db_open_check(n, L, pitch, opts, db, false);
+    require_device();
+    InterruptScope sigint;
+    ResidentDb *h;
+    if (opts && opts->packed_input) {
+      h = db_open(dev_seqs, n, L, pitch, nullptr, 0);
+    } else {  // ASCII rows are encoded once into 4-bit rows the handle owns (db.inl: one pack for both sides)
+      DevBuf<uint8_t> nib;
+      const size_t pitch4 = packed_pitch(L);
+      nib.alloc(n * pitch4);
+      encode_rows_device(dev_seqs, n, L, pitch, nib.p, pitch4, 0);
+      const uint8_t *rows = nib.p;
+      h = db_open(rows, n, L, pitch4, &nib, 0);
+    }
+    db_register(h);
+    *db = h;
+  });
+}
+
+int tracs_db_query_host(void *db, const uint8_t *seqs, size_t nq, size_t pitch, const tracs_opts_t *opts, tracs_edges_t *out) {
+  if (out) memset(out, 0, sizeof *out);
+  memset(&g_stats, 0, sizeof g_stats);
+  return guarded([&] {
+    ResidentDb *h = nullptr;
+    uint64_t L = 0;
+    tracs_opts_t o = db_query_check(db, nq, pitch, opts, out, true, h, L);
+    require_device();
+    InterruptScope sigint;
+    HostEdges he;
+    if (nq > 0) {
+      DevBuf<uint8_t> nib;
+      size_t pitch4 = 0;
+      stream_host_to_packed(seqs, nq, L, pitch, o.packed_input != 0, nib, pitch4, 0);
+      db_query(*h, nib.p, nq, pitch4, o, he, 0);
+    }
+    finish_edges(he, o, nq, L, out, 0);
+  });
+}
+
+int tracs_db_query_device(void *db, const uint8_t *dev_seqs, size_t nq, size_t pitch, const tracs_opts_t *opts, tracs_edges_t *out) {
+  if (out) memset(out, 0, sizeof *out);
+  memset(&g_stats, 0, sizeof g_stats);
+  return guarded([&] {
+    ResidentDb *h = nullptr;
+    uint64_t L = 0;
+    tracs_opts_t o = db_query_check(db, nq, pitch, opts, out, false, h, L);
+    require_device();
+    InterruptScope sigint;
+    HostEdges he;
+    DevBuf<uint8_t> nib;
+    size_t qpitch = pitch;
+    if (!o.packed_input && nq > 0) {
+      qpitch = packed_pitch(L);
+      nib.alloc(nq * qpitch);
+      encode_rows_device(dev_seqs, nq, L, pitch, nib.p, qpitch, 0);
+    }
+    db_query(*h, o.packed_input ? dev_seqs : nib.p, nq, qpitch, o, he, 0);
+    finish_edges(he, o, nq, L, out, 0);
+  });
+}
+
+int tracs_db_info(void *db, tracs_db_info_t *out) {
+  return guarded([&] {
+    if (!out) throw std::runtime_error("database info: out is NULL");
+    db_info(*db_lookup(db), *out);
+  });
+}
+
+int tracs_db_close(void *db) {
+  return guarded([&] {
+    ResidentDb *h = db_lookup(db);
+    {
+      std::lock_guard<std::mutex> g(g_db_mu);
+      g_db_live.erase(h);
+    }
+    db_close(h);
   });
 }
 

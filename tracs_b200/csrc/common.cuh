@@ -84,6 +84,7 @@ template <typename T>
 struct DevBuf {
   T *p = nullptr;
   size_t n = 0;
+  bool owned = true;
   DevBuf() {}
   explicit DevBuf(size_t count) { alloc(count); }
   DevBuf(const DevBuf &) = delete;
@@ -93,10 +94,18 @@ struct DevBuf {
     n = count;
     if (count) p = (T *)dev_cache_alloc(count * sizeof(T));
   }
+  // a view of `count` elements of memory that something else owns: never freed through this object
+  void borrow(T *q, size_t count) {
+    release();
+    p = q;
+    n = count;
+    owned = false;
+  }
   void release() {
-    if (p) dev_cache_free(p);
+    if (p && owned) dev_cache_free(p);
     p = nullptr;
     n = 0;
+    owned = true;
   }
   ~DevBuf() { release(); }
 };
@@ -310,6 +319,14 @@ void sweep_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint64_t pitc
 // every pair's distance into a dense int32 device matrix (tracs_distance_matrix_device; arguments validated by the caller)
 void distance_matrix_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint64_t pitch, const tracs_opts_t &o, int32_t *out,
                             uint64_t ld, cudaStream_t st);
+
+// resident sample database (db.inl; arguments validated by the caller; database and query rows 4-bit). db_open takes over
+// `adopt` (the rows it points into) when given; otherwise the rows stay the caller's.
+struct ResidentDb;
+ResidentDb *db_open(const uint8_t *dev_rows, uint64_t n, uint64_t L, uint64_t pitch, DevBuf<uint8_t> *adopt, cudaStream_t st);
+void db_query(ResidentDb &db, const uint8_t *dev_q, uint64_t nq, uint64_t qpitch, const tracs_opts_t &o, HostEdges &out, cudaStream_t st);
+void db_info(const ResidentDb &db, tracs_db_info_t &out);
+void db_close(ResidentDb *db);
 
 // last step of the site-sharded sweep (shard.inl): summed candidate vectors -> edge columns
 void site_shard_finish_device(const uint64_t *dev_keys, const uint32_t *dev_d, const uint32_t *dev_union, uint64_t n_keys, uint64_t n,

@@ -1369,8 +1369,11 @@ __global__ void k_sum_u32(const uint32_t *__restrict__ v, uint64_t n, unsigned l
 
 // ASCII matrix (device) -> N-plane + summaries + variable-site bit-planes (K0a + K0b)
 // `packed`: dev_seqs holds 4-bit masks, two sites per byte (pack4.inl), pitch in bytes
+// `rows_before`: the N-plane, its summary and the N counts get that many unused (zeroed-summary) rows before sample 0,
+// which g.nplane.p etc. then point at (the resident database, db.inl, packs query rows there). `keep_colmask`: receives
+// the column AND of the 4-bit masks (L / 8 words).
 static void ingest_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint64_t pitch, bool packed, bool keep_site_idx,
-                          Ingested &g, cudaStream_t st) {
+                          Ingested &g, cudaStream_t st, uint64_t rows_before = 0, DevBuf<uint32_t> *keep_colmask = nullptr) {
   tracs_stats_t &S = g_stats;
   if (!packed && (pitch % 32 != 0 || pitch < round_up(L, 32)))
     throw std::runtime_error("device alignment pitch must be a multiple of 32 and >= L rounded up to 32");
@@ -1402,15 +1405,17 @@ static void ingest_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint6
   const char *nb_env = getenv("TRACS_NBLOCKS");
   const bool sparse_candidate = early && !(np_env && !strcmp(np_env, "always")) && !(nb_env && !strcmp(nb_env, "dense"));
   g.nplane_sparse = false;
-  nplane.alloc(n * npitch);
-  nsum.alloc(n * spitch);
-  ncount.alloc(n);
+  nplane.alloc((rows_before + n) * npitch);
+  nsum.alloc((rows_before + n) * spitch);
+  ncount.alloc(rows_before + n);
+  uint32_t *const np0 = nplane.p + rows_before * npitch, *const nc0 = ncount.p + rows_before;
+  uint8_t *const ns0 = nsum.p + rows_before * spitch;
   const uint32_t Npad = (uint32_t)round_up(n, TILE);
   DevBuf<uint32_t> &site_idx = g.site_idx;
   T.start();
   TRACS_CK(cudaMemsetAsync(colmask.p, 0xFF, colmask.n * sizeof(uint32_t), st));
   TRACS_CK(cudaMemsetAsync(nsum.p, 0, nsum.n, st));
-  TRACS_CK(cudaMemsetAsync(ncount.p, 0, n * sizeof(uint32_t), st));
+  TRACS_CK(cudaMemsetAsync(ncount.p, 0, ncount.n * sizeof(uint32_t), st));
 
   // variable-site list from the column AND: flags -> select; returns the count (synchronises the stream)
   auto select_sites = [&](DevBuf<uint32_t> &list) -> uint64_t {
@@ -1435,27 +1440,27 @@ static void ingest_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint6
     if (packed) {
       if (VE && g.nplane_sparse) {
         TRACS_CK(cudaFuncSetAttribute((k_pack4<true, true>), cudaFuncAttributePreferredSharedMemoryCarveout, 60));
-        k_pack4<true, true><<<grid, PACK_THREADS, 0, st>>>(dev_seqs, sa, sb, L, pitch, colmask.p, nplane.p, npitch, nsum.p, spitch,
-                                                         ncount.p, elist, VE, X, XP);
+        k_pack4<true, true><<<grid, PACK_THREADS, 0, st>>>(dev_seqs, sa, sb, L, pitch, colmask.p, np0, npitch, ns0, spitch,
+                                                         nc0, elist, VE, X, XP);
       } else if (VE) {
         TRACS_CK(cudaFuncSetAttribute((k_pack4<true, false>), cudaFuncAttributePreferredSharedMemoryCarveout, 60));
-        k_pack4<true><<<grid, PACK_THREADS, 0, st>>>(dev_seqs, sa, sb, L, pitch, colmask.p, nplane.p, npitch, nsum.p, spitch, ncount.p,
+        k_pack4<true><<<grid, PACK_THREADS, 0, st>>>(dev_seqs, sa, sb, L, pitch, colmask.p, np0, npitch, ns0, spitch, nc0,
                                                    elist, VE, X, XP);
       } else {
-        k_pack4<false><<<grid, PACK_THREADS, 0, st>>>(dev_seqs, sa, sb, L, pitch, colmask.p, nplane.p, npitch, nsum.p, spitch, ncount.p,
+        k_pack4<false><<<grid, PACK_THREADS, 0, st>>>(dev_seqs, sa, sb, L, pitch, colmask.p, np0, npitch, ns0, spitch, nc0,
                                                     nullptr, 0, nullptr, 0);
       }
     } else if (VE) {
       TRACS_CK(cudaFuncSetAttribute(k_pack_x<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 60));  // 3 x 34 KB per SM (per device)
       TRACS_CK(cudaFuncSetAttribute(k_pack_x<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 60));
       if (g.nplane_sparse)
-        k_pack_x<true><<<grid, PACK_THREADS, 0, st>>>(dev_seqs, sa, sb, L, pitch, colmask.p, nplane.p, npitch, nsum.p, spitch, ncount.p,
+        k_pack_x<true><<<grid, PACK_THREADS, 0, st>>>(dev_seqs, sa, sb, L, pitch, colmask.p, np0, npitch, ns0, spitch, nc0,
                                                     elist, VE, X, XP);
       else
-        k_pack_x<false><<<grid, PACK_THREADS, 0, st>>>(dev_seqs, sa, sb, L, pitch, colmask.p, nplane.p, npitch, nsum.p, spitch, ncount.p,
+        k_pack_x<false><<<grid, PACK_THREADS, 0, st>>>(dev_seqs, sa, sb, L, pitch, colmask.p, np0, npitch, ns0, spitch, nc0,
                                                      elist, VE, X, XP);
     } else {
-      k_pack<<<grid, PACK_THREADS, 0, st>>>(dev_seqs, sa, sb, L, pitch, colmask.p, nplane.p, npitch, nsum.p, spitch, ncount.p);
+      k_pack<<<grid, PACK_THREADS, 0, st>>>(dev_seqs, sa, sb, L, pitch, colmask.p, np0, npitch, ns0, spitch, nc0);
     }
     S.kernel_launches++;
     TRACS_CK(cudaGetLastError());
@@ -1474,7 +1479,7 @@ static void ingest_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint6
     launch_pack(0, n_first, nullptr, 0, nullptr, 0);
     std::vector<uint32_t> first_cnt(sparse_candidate ? n_first : 0);
     if (sparse_candidate)  // lands with the synchronisation inside select_sites
-      TRACS_CK(cudaMemcpyAsync(first_cnt.data(), ncount.p, n_first * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+      TRACS_CK(cudaMemcpyAsync(first_cnt.data(), nc0, n_first * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     VE = select_sites(elist);
     if (VE > L / 16) VE = 0;  // very diverse alignment: the scattered pass reads dense lines anyway
     if (VE) {
@@ -1550,7 +1555,7 @@ static void ingest_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint6
     TRACS_CK(cudaGetLastError());
     DevBuf<unsigned long long> ntot(1);
     TRACS_CK(cudaMemsetAsync(ntot.p, 0, 8, st));
-    k_sum_u32<<<64, 256, 0, st>>>(ncount.p, n, ntot.p);
+    k_sum_u32<<<64, 256, 0, st>>>(nc0, n, ntot.p);
     S.kernel_launches++;
     uint32_t h_amb = 0;
     unsigned long long h_ntot = 0;
@@ -1563,6 +1568,10 @@ static void ingest_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint6
   }
   S.ms_compact += T.stop();
   if (!keep_site_idx) site_idx.release();
+  if (keep_colmask) {
+    std::swap(keep_colmask->p, colmask.p);
+    std::swap(keep_colmask->n, colmask.n);
+  }
 }
 
 // Fused transmission likelihood (K3) for a sorted device edge list: dense table over (d, day difference).
@@ -2084,22 +2093,12 @@ static void sweep_banded(const Ingested &g, const TilePlan &plan, SweepArgs a, b
   }
 }
 
-// Sweeps the device-resident ASCII matrix and appends edges (sorted) to `out`.
-void sweep_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint64_t pitch, const tracs_opts_t &o,
-                  HostEdges &out, cudaStream_t st) {
+// The pair sweep of an ingested alignment over the range of `o` (i_end already clipped to ing.n): tile plan, filter-and-refine
+// or banded full-length sweep, sorted edges appended to `out`.
+static void sweep_ingested(const Ingested &ing, const tracs_opts_t &o, uint64_t i_end, uint64_t j_start, HostEdges &out,
+                           cudaStream_t st) {
   tracs_stats_t &S = g_stats;
-  S.n_samples = n;
-  S.seq_length = L;
-  const uint64_t i_end = std::min<uint64_t>(o.i_end, n);
-  const uint64_t j_start = o.j_start;
-  if (n == 0 || i_end == 0 || j_start >= n) return;
-  if (n >= (1ull << 31)) throw std::runtime_error("too many samples");
-  Timer Ttot(st);
-  Ttot.start();
-
-  // ---- ingest + plan ------------------------------------------------------------------------
-  Ingested ing;
-  ingest_device(dev_seqs, n, L, pitch, o.packed_input != 0, o.filter != 0, ing, st);
+  const uint64_t n = ing.n;
   const int world = std::max(1, (int)o.shard_world), rank = std::max(0, (int)o.shard_rank);
   const TilePlan plan = plan_tiles(n, i_end, j_start, ing.Npad, rank, world);
   uint64_t total_pairs = 0, total_tiles = 0;
@@ -2108,10 +2107,7 @@ void sweep_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint64_t pitc
     total_tiles += plan.n_cb - std::max(plan.my_rb[k], plan.cb_min);
   }
   S.n_pairs += total_pairs;
-  if (plan.my_rb.empty()) {
-    S.ms_total = Ttot.stop();
-    return;
-  }
+  if (plan.my_rb.empty()) return;
   const bool tc_ok = use_tensor_cores(o, ing);
   // A thresholded call first tries filter-and-refine over ALL owned row-blocks in one launch per window (the candidate
   // list is bounded: only a few per cent of the pairs may survive); otherwise, or when the prefilter is not selective,
@@ -2132,6 +2128,23 @@ void sweep_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint64_t pitc
     done = sweep_prefiltered(ing, plan, total_pairs, a, tc_ok, end_bit, o, fuse_trans ? &lut : nullptr, out, st);
   }
   if (!done) sweep_banded(ing, plan, a, tc_ok, end_bit, o, fuse_trans ? &lut : nullptr, out, st);
+}
+
+// Sweeps the device-resident ASCII matrix and appends edges (sorted) to `out`.
+void sweep_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uint64_t pitch, const tracs_opts_t &o,
+                  HostEdges &out, cudaStream_t st) {
+  tracs_stats_t &S = g_stats;
+  S.n_samples = n;
+  S.seq_length = L;
+  const uint64_t i_end = std::min<uint64_t>(o.i_end, n);
+  const uint64_t j_start = o.j_start;
+  if (n == 0 || i_end == 0 || j_start >= n) return;
+  if (n >= (1ull << 31)) throw std::runtime_error("too many samples");
+  Timer Ttot(st);
+  Ttot.start();
+  Ingested ing;
+  ingest_device(dev_seqs, n, L, pitch, o.packed_input != 0, o.filter != 0, ing, st);
+  sweep_ingested(ing, o, i_end, j_start, out, st);
   S.ms_total = Ttot.stop();
 }
 
@@ -2170,4 +2183,5 @@ void distance_matrix_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uin
 }  // namespace tracs
 
 #include "shard.inl"
+#include "db.inl"
 #include "tc_peak.inl"

@@ -89,21 +89,27 @@ def distance(msa_files, output_file, msa_db=None, metadata=None, snp_threshold=2
         for msa in msa_files:
             fastas = [msa, msa_db] if msa_db is not None else [msa]
             rows, cols, snp, names, filt, ncomp = api.pairsnp(fasta=fastas, n_threads=n_cpu, dist=snp_threshold, filter=recomb_filter)
-            ref = os.path.basename(msa).split(".")[0].replace("_combined", "")  # tracs/distance.py:208-209
-            if dates is not None and len(rows) > 0:
-                dt = date_differences(rows, cols, names, dates)
-                # with the filter on, the likelihood is fed the filtered distance (tracs/distance.py:182-192)
-                p0, eK = api.trans_dist(filt if recomb_filter else snp, dt, clock_rate, trans_rate, precision)
-                p0 = np.exp(np.asarray(p0))  # tracs/transcluster.py:38-39
-                filt_col = filt if recomb_filter else ["NA"] * len(rows)  # tracs/distance.py:204
-                for e in range(len(rows)):
-                    if trans_threshold is None or trans_threshold >= eK[e]:  # tracs/distance.py:222
-                        out.write(",".join([names[rows[e]], names[cols[e]], str(dt[e]), str(int(snp[e])), str(p0[e]), str(eK[e]),
-                                            str(filt_col[e]), str(ncomp[e]), ref]) + "\n")
-            else:
-                for e in range(len(rows)):  # tracs/distance.py:239-258
-                    out.write(",".join([names[rows[e]], names[cols[e]], "NA", str(int(snp[e])), "NA", "NA", str(filt[e]), str(ncomp[e]),
-                                        ref]) + "\n")
+            write_rows(out, msa, rows, cols, snp, names, filt, ncomp, dates, recomb_filter, clock_rate, trans_rate, trans_threshold,
+                       precision)
+
+
+def write_rows(out, msa, rows, cols, snp, names, filt, ncomp, dates, recomb_filter, clock_rate, trans_rate, trans_threshold, precision):
+    """The CSV rows of one MSA's edge lists (lists, in (row, col) order; names indexed by rows / cols) into the open file."""
+    ref = os.path.basename(msa).split(".")[0].replace("_combined", "")  # tracs/distance.py:208-209
+    if dates is not None and len(rows) > 0:
+        dt = date_differences(rows, cols, names, dates)
+        # with the filter on, the likelihood is fed the filtered distance (tracs/distance.py:182-192)
+        p0, eK = api.trans_dist(filt if recomb_filter else snp, dt, clock_rate, trans_rate, precision)
+        p0 = np.exp(np.asarray(p0))  # tracs/transcluster.py:38-39
+        filt_col = filt if recomb_filter else ["NA"] * len(rows)  # tracs/distance.py:204
+        for e in range(len(rows)):
+            if trans_threshold is None or trans_threshold >= eK[e]:  # tracs/distance.py:222
+                out.write(",".join([names[rows[e]], names[cols[e]], str(dt[e]), str(int(snp[e])), str(p0[e]), str(eK[e]),
+                                    str(filt_col[e]), str(ncomp[e]), ref]) + "\n")
+    else:
+        for e in range(len(rows)):  # tracs/distance.py:239-258
+            out.write(",".join([names[rows[e]], names[cols[e]], "NA", str(int(snp[e])), "NA", "NA", str(filt[e]), str(ncomp[e]),
+                                ref]) + "\n")
 
 
 def main(argv=None):
