@@ -14,6 +14,13 @@
 // delta <= 0 (same-day samples): the shipped -ffast-math reference never leaves the k loop and
 // converges to the negative-binomial mean (N+1)*beta/lamb while over-reading its lgamma table
 // (SURVEY F6). That closed form is returned here.
+//
+// Samples far apart (SURVEY F7): the reference stops the E[K] series once upper_bound_E - sum_k t_k <= thr. The bound grows
+// like e^{delta lamb}; once 2^-32 of it exceeds thr the difference is rounding noise and the reference returns a partial
+// sum that can be any fraction of E[K] (0.138 for 148.38 two years apart at the default rates). On those keys the loop
+// stops on the geometric tail bound of the t_k instead (trans.cuh); the other keys keep the reference's rule and values.
+// A series not converged by the reference's cap of k = 10000 returns E[K] = +inf instead of a truncated sum.
+// A threshold <= 0 or NaN asks for E[K] to working precision: the tail bound is then compared with 2^-52 of the sum.
 #include <math.h>
 
 #include <memory>
