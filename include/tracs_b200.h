@@ -173,7 +173,18 @@ int tracs_write_distance_matrix(const char *path, const int32_t *m, size_t rows,
  *   and unchanged while the handle is open (the library only reads it; a second copy of a 100 GB database would not fit).
  *   _device with ASCII rows encodes them once into 4-bit rows the library owns (half their size); dev_seqs is not kept.
  * The handle belongs to the device that was current at open; a query while another device is current fails. Closing a handle
- * twice, or passing one that was never opened, fails without touching memory. */
+ * twice, or passing one that was never opened, fails without touching memory.
+ *
+ * append: adds a batch b (m samples, the same L) to the database and returns the edges it brings:
+ *   tracs_db_append_*(db, b, opts)  returns exactly what  tracs_pairsnp_host([db; b], opts with i_end = 0, j_start = n_db)
+ * returns: every pair with a sample in the batch (batch x database and batch x batch), every column, the same (row, col)
+ * order, indices of the grown collection (the batch is n_db .. n_db + m - 1). opts, input forms and refusals as for the query
+ * (the messages start "database append: "); days holds n_db + m values, the database first. Afterwards the database is
+ * [db; b]: info n grows by m, n_variable_sites by the sites the batch makes variable (new_sites), and every later query or
+ * append returns what it returns on a database opened on [db; b]. An append that fails (its bit-planes or the grown buffers do
+ * not fit: the message gives the size in GB; SIGINT: status 4; any other error) leaves the database as it was. Appended rows
+ * are kept in device memory the library owns; a borrowed buffer is still never written. The N-plane grows to 1.25x the
+ * database's rows when the room behind it runs out (the old and the new N-plane are both held while the rows are copied). */
 typedef struct tracs_db_info {
   uint64_t n;                /* database samples                                                   */
   uint64_t L;                /* sites                                                              */
@@ -182,12 +193,15 @@ typedef struct tracs_db_info {
   int32_t reserved0;
   uint64_t bytes_held;       /* device bytes the handle holds (borrowed rows not counted)          */
   uint64_t query_rows;       /* query rows swept at once; larger batches go through in chunks       */
-  uint64_t new_sites;        /* sites variable in [q; db] but not in db, for the last query batch  */
+  uint64_t new_sites;        /* sites variable in [q; db] but not in db, for the last query or
+                                appended batch                                                     */
 } tracs_db_info_t;
 int tracs_db_open_host(const uint8_t *seqs, size_t n, size_t L, size_t pitch, const tracs_opts_t *opts, void **db);
 int tracs_db_open_device(const uint8_t *dev_seqs, size_t n, size_t L, size_t pitch, const tracs_opts_t *opts, void **db);
 int tracs_db_query_host(void *db, const uint8_t *seqs, size_t nq, size_t pitch, const tracs_opts_t *opts, tracs_edges_t *out);
 int tracs_db_query_device(void *db, const uint8_t *dev_seqs, size_t nq, size_t pitch, const tracs_opts_t *opts, tracs_edges_t *out);
+int tracs_db_append_host(void *db, const uint8_t *seqs, size_t m, size_t pitch, const tracs_opts_t *opts, tracs_edges_t *out);
+int tracs_db_append_device(void *db, const uint8_t *dev_seqs, size_t m, size_t pitch, const tracs_opts_t *opts, tracs_edges_t *out);
 int tracs_db_info(void *db, tracs_db_info_t *out);
 int tracs_db_close(void *db);
 

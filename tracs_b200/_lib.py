@@ -64,7 +64,7 @@ SYMBOLS = ["tracs_pairsnp", "tracs_pairsnp_host", "tracs_pairsnp_device", "tracs
            "tracs_write_distance_csv", "tracs_float_repr", "tracs_pairsnp_packed", "tracs_encode_packed", "tracs_site_shard_finish", "tracs_tc_peak", "tracs_tc_peak_sustained", "tracs_site_shard_select", "tracs_site_shard_emit",
            "tracs_host_register", "tracs_host_unregister", "tracs_distance_matrix_device", "tracs_distance_matrix_host",
            "tracs_write_distance_matrix", "tracs_db_open_host", "tracs_db_open_device", "tracs_db_query_host", "tracs_db_query_device",
-           "tracs_db_info", "tracs_db_close"]
+           "tracs_db_append_host", "tracs_db_append_device", "tracs_db_info", "tracs_db_close"]
 
 _lib = None
 
@@ -128,6 +128,8 @@ def lib():
         L.tracs_db_open_device.argtypes = [C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.POINTER(Opts), C.POINTER(C.c_void_p)]
         L.tracs_db_query_host.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.POINTER(Opts), C.POINTER(Edges)]
         L.tracs_db_query_device.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.POINTER(Opts), C.POINTER(Edges)]
+        L.tracs_db_append_host.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.POINTER(Opts), C.POINTER(Edges)]
+        L.tracs_db_append_device.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.POINTER(Opts), C.POINTER(Edges)]
         L.tracs_db_info.argtypes = [C.c_void_p, C.POINTER(DbInfo)]
         L.tracs_db_close.argtypes = [C.c_void_p]
         _lib = L

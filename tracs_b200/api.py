@@ -226,6 +226,10 @@ class Database:
     same order, rows = query index in [0, nq), cols = nq + database index. `days` (for the transmission likelihood) covers
     the queries first, then the database. Not supported: the recombination filter, query x query pairs.
 
+    append(b) adds the batch to the database and returns exactly what pairsnp_matrix(concatenate([db, b]), j_start=n_db)
+    returns: every pair with a sample in the batch, indexed in the grown collection (the batch is n_db .. n_db + m - 1).
+    Afterwards the database is [db; b]; an append that raises leaves it as it was.
+
     Database(seqs) copies a host matrix (ASCII uint8[n][L], or pack_nibbles rows with packed=True and L) into device memory
     the handle owns. Use it as a context manager, or close() it, to release that memory."""
 
@@ -294,9 +298,50 @@ class Database:
         _lib.check(_lib.lib().tracs_db_query_device(C.c_void_p(self._handle()), C.c_void_p(ptr), int(nq), int(pitch), C.byref(o), C.byref(e)))
         return _lib.take_edges(e, names=False)
 
+    def _append_opts(self, dist, days, want_ncomp, full_sweep, packed, m, names):
+        if days is not None and len(days) != self.n + m:
+            raise ValueError("days must hold n_db + m = %d values (the database first, then the batch)" % (self.n + m))
+        if self.names is not None and (names is None or len(names) != m):
+            raise ValueError("the database has sample names: give one name per appended sample (%d)" % m)
+        if self.names is None and names is not None:
+            raise ValueError("the database has no sample names to extend")
+        return make_opts(dist=dist, days=days, want_ncomp=want_ncomp, full_sweep=full_sweep, packed=packed)
+
+    def _appended(self, e, m, names):
+        r = _lib.take_edges(e, names=False)
+        self.n += m
+        if names is not None:
+            self.names = self.names + list(names)
+        return r
+
+    def append(self, seqs, dist=INT32_MAX, days=None, want_ncomp=True, full_sweep=False, packed=False, L=None, names=None):
+        """Adds the HOST rows (ASCII uint8[m][L], or pack_nibbles rows with packed=True) to the database and returns the edges
+        of every pair with a sample in the batch, as the dict of pairsnp_matrix, indexed in the grown collection. `days`:
+        n_db + m values, the database first. `names`: one per appended sample, required when the database has names
+        (from_fasta), which it then extends."""
+        seqs = np.ascontiguousarray(seqs, dtype=np.uint8)
+        if seqs.ndim != 2:
+            raise ValueError("seqs must be a 2-D uint8 matrix")
+        m, width = seqs.shape
+        L = (width if not packed else self.L) if L is None else int(L)
+        if L != self.L:
+            raise ValueError("appended L (%d sites) differs from the database's L (%d sites)" % (L, self.L))
+        o, keep = self._append_opts(dist, days, want_ncomp, full_sweep, packed, m, names)
+        e = Edges()
+        _lib.check(_lib.lib().tracs_db_append_host(C.c_void_p(self._handle()), seqs.ctypes.data, m, width, C.byref(o), C.byref(e)))
+        return self._appended(e, m, names)
+
+    def append_device(self, ptr, m, pitch, dist=INT32_MAX, days=None, want_ncomp=True, full_sweep=False, packed=False, names=None):
+        """append() of DEVICE rows (raw pointer as int; ASCII rows, or 4-bit rows with packed=True) of the database's L. The
+        rows are copied: the buffer is not kept."""
+        o, keep = self._append_opts(dist, days, want_ncomp, full_sweep, packed, int(m), names)
+        e = Edges()
+        _lib.check(_lib.lib().tracs_db_append_device(C.c_void_p(self._handle()), C.c_void_p(ptr), int(m), int(pitch), C.byref(o), C.byref(e)))
+        return self._appended(e, int(m), names)
+
     def info(self):
         """n, L, n_variable_sites (of the database), device, bytes_held, query_rows (swept at once) and new_sites (sites
-        that the last query batch made variable)."""
+        that the last query or appended batch made variable)."""
         i = _lib.DbInfo()
         _lib.check(_lib.lib().tracs_db_info(C.c_void_p(self._handle()), C.byref(i)))
         return i.as_dict()

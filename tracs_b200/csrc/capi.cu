@@ -847,10 +847,10 @@ static void db_register(ResidentDb *db) {
   g_db_live.insert(db);
 }
 
-// Argument check of tracs_db_query_*. Host code only, so it runs before require_device().
-static tracs_opts_t db_query_check(void *h, size_t nq, size_t pitch, const tracs_opts_t *opts, const tracs_edges_t *out, bool host_input,
-                                   ResidentDb *&db, uint64_t &L) {
-  const char *pre = "database query: ";
+// Argument check of tracs_db_query_* and (append) tracs_db_append_*. Host code only, so it runs before require_device().
+static tracs_opts_t db_query_check(bool append, void *h, size_t nq, size_t pitch, const tracs_opts_t *opts, const tracs_edges_t *out,
+                                   bool host_input, ResidentDb *&db, uint64_t &L) {
+  const char *pre = append ? "database append: " : "database query: ";
   if (!out) throw std::runtime_error(std::string(pre) + "out is NULL");
   tracs_opts_t o;
   if (opts) o = *opts; else { memset(&o, 0, sizeof o); o.dist = INT32_MAX; o.want_ncomp = 1; }
@@ -858,9 +858,10 @@ static tracs_opts_t db_query_check(void *h, size_t nq, size_t pitch, const tracs
   if (o.keep_on_device) throw std::runtime_error(std::string(pre) + "opts->keep_on_device is not supported against a database");
   if (o.shard_world > 1) throw std::runtime_error(std::string(pre) + "opts->shard_world > 1: a database is swept on one GPU");
   if (o.i_end || o.j_start)
-    throw std::runtime_error(std::string(pre) + "opts->i_end / opts->j_start must be 0: rows are the queries, cols the database");
+    throw std::runtime_error(std::string(pre) + "opts->i_end / opts->j_start must be 0: " +
+                             (append ? "every pair with a sample in the batch is returned" : "rows are the queries, cols the database"));
   if (o.sweep_variant < 0 || o.sweep_variant > 2) throw std::runtime_error(std::string(pre) + "opts->sweep_variant must be 0, 1 or 2");
-  if (nq >= (1ull << 31)) throw std::runtime_error(std::string(pre) + "nq: too many samples");
+  if (nq >= (1ull << 31)) throw std::runtime_error(std::string(pre) + (append ? "m" : "nq") + ": too many samples");
   db = db_lookup(h);
   tracs_db_info_t info;
   db_info(*db, info);
@@ -927,7 +928,7 @@ int tracs_db_query_host(void *db, const uint8_t *seqs, size_t nq, size_t pitch, 
   return guarded([&] {
     ResidentDb *h = nullptr;
     uint64_t L = 0;
-    tracs_opts_t o = db_query_check(db, nq, pitch, opts, out, true, h, L);
+    tracs_opts_t o = db_query_check(false, db, nq, pitch, opts, out, true, h, L);
     require_device();
     InterruptScope sigint;
     HostEdges he;
@@ -947,7 +948,7 @@ int tracs_db_query_device(void *db, const uint8_t *dev_seqs, size_t nq, size_t p
   return guarded([&] {
     ResidentDb *h = nullptr;
     uint64_t L = 0;
-    tracs_opts_t o = db_query_check(db, nq, pitch, opts, out, false, h, L);
+    tracs_opts_t o = db_query_check(false, db, nq, pitch, opts, out, false, h, L);
     require_device();
     InterruptScope sigint;
     HostEdges he;
@@ -960,6 +961,44 @@ int tracs_db_query_device(void *db, const uint8_t *dev_seqs, size_t nq, size_t p
     }
     db_query(*h, o.packed_input ? dev_seqs : nib.p, nq, qpitch, o, he, 0);
     finish_edges(he, o, nq, L, out, 0);
+  });
+}
+
+int tracs_db_append_host(void *db, const uint8_t *seqs, size_t m, size_t pitch, const tracs_opts_t *opts, tracs_edges_t *out) {
+  if (out) memset(out, 0, sizeof *out);
+  memset(&g_stats, 0, sizeof g_stats);
+  return guarded([&] {
+    ResidentDb *h = nullptr;
+    uint64_t L = 0;
+    const tracs_opts_t o = db_query_check(true, db, m, pitch, opts, out, true, h, L);
+    require_device();
+    InterruptScope sigint;
+    HostEdges he;
+    DevBuf<uint8_t> nib;
+    size_t pitch4 = packed_pitch(L);
+    if (m > 0) stream_host_to_packed(seqs, m, L, pitch, o.packed_input != 0, nib, pitch4, 0);
+    db_append(*h, nib.p, m, pitch4, o, he, [&] { finish_edges(he, o, m, L, out, 0); }, 0);
+  });
+}
+
+int tracs_db_append_device(void *db, const uint8_t *dev_seqs, size_t m, size_t pitch, const tracs_opts_t *opts, tracs_edges_t *out) {
+  if (out) memset(out, 0, sizeof *out);
+  memset(&g_stats, 0, sizeof g_stats);
+  return guarded([&] {
+    ResidentDb *h = nullptr;
+    uint64_t L = 0;
+    const tracs_opts_t o = db_query_check(true, db, m, pitch, opts, out, false, h, L);
+    require_device();
+    InterruptScope sigint;
+    HostEdges he;
+    DevBuf<uint8_t> nib;
+    size_t bpitch = pitch;
+    if (!o.packed_input && m > 0) {
+      bpitch = packed_pitch(L);
+      nib.alloc(m * bpitch);
+      encode_rows_device(dev_seqs, m, L, pitch, nib.p, bpitch, 0);
+    }
+    db_append(*h, o.packed_input ? dev_seqs : nib.p, m, bpitch, o, he, [&] { finish_edges(he, o, m, L, out, 0); }, 0);
   });
 }
 

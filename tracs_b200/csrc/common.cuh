@@ -6,6 +6,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <sys/mman.h>
+#include <functional>
 #include <memory>
 #include <new>
 #include <stdexcept>
@@ -325,6 +326,10 @@ void distance_matrix_device(const uint8_t *dev_seqs, uint64_t n, uint64_t L, uin
 struct ResidentDb;
 ResidentDb *db_open(const uint8_t *dev_rows, uint64_t n, uint64_t L, uint64_t pitch, DevBuf<uint8_t> *adopt, cudaStream_t st);
 void db_query(ResidentDb &db, const uint8_t *dev_q, uint64_t nq, uint64_t qpitch, const tracs_opts_t &o, HostEdges &out, cudaStream_t st);
+// db_append: the edges of the batch b against [db; b] into `out`; `finish` (the caller's result) runs before the append is
+// committed, and an exception from either leaves the database as it was
+void db_append(ResidentDb &db, const uint8_t *dev_b, uint64_t m, uint64_t bpitch, const tracs_opts_t &o, HostEdges &out,
+               const std::function<void()> &finish, cudaStream_t st);
 void db_info(const ResidentDb &db, tracs_db_info_t &out);
 void db_close(ResidentDb *db);
 

@@ -2,7 +2,11 @@
 
 The database FASTA is read and ingested on the GPU once (tracs_b200.Database); every --msa file is then swept against it
 as the two-file call `python -m tracs_b200.distance --msa q.fasta --msa-db db.fasta` would sweep it, and the output CSV
-is byte-identical to what that command writes with the same options (rows are written by the same code)."""
+is byte-identical to what that command writes with the same options (rows are written by the same code).
+
+With --append, each --msa file is placed and then added to the database, so later files are also compared with earlier ones:
+the rows of a file are every pair whose later sample is in that file (against the database, the earlier files and the file
+itself), as `python -m tracs_b200.distance --msa` on the concatenation of the database and the files lists them."""
 import argparse
 import sys
 
@@ -11,7 +15,7 @@ from .distance import HEADER, read_dates, write_rows
 
 
 def query(db_file, msa_files, output_file, metadata=None, snp_threshold=2147483647, clock_rate=1e-3 * 29903, trans_rate=73.0,
-          trans_threshold=None, precision=0.01, n_cpu=1):
+          trans_threshold=None, precision=0.01, n_cpu=1, append=False):
     dates = read_dates(metadata) if metadata is not None else None
     with api.Database.from_fasta(db_file, n_threads=n_cpu) as db, open(output_file, "w") as out:
         out.write(HEADER)
@@ -20,8 +24,13 @@ def query(db_file, msa_files, output_file, metadata=None, snp_threshold=21474836
             if seqs.shape[1] != db.L:
                 raise ValueError("%s: sequences of %d sites, the database %s has %d: the alignments must have the same length"
                                  % (msa, seqs.shape[1], db_file, db.L))
-            r = db.query(seqs, dist=snp_threshold)
-            write_rows(out, msa, r["rows"].tolist(), r["cols"].tolist(), r["dist"].tolist(), names + db.names, r["filt"].tolist(),
+            if append:
+                r = db.append(seqs, dist=snp_threshold, names=names)
+                all_names = db.names
+            else:
+                r = db.query(seqs, dist=snp_threshold)
+                all_names = names + db.names
+            write_rows(out, msa, r["rows"].tolist(), r["cols"].tolist(), r["dist"].tolist(), all_names, r["filt"].tolist(),
                        r["ncomp"].tolist(), dates, False, clock_rate, trans_rate, trans_threshold, precision)
 
 
@@ -38,6 +47,8 @@ def main(argv=None):
     ap.add_argument("-K", "--trans_threshold", type=float, default=None)
     ap.add_argument("--precision", type=float, default=0.01)
     ap.add_argument("-t", "--threads", dest="n_cpu", type=int, default=1)
+    ap.add_argument("--append", action="store_true", help="add each --msa file to the database after placing it, so that later "
+                                                          "files are also compared with it")
     a = ap.parse_args(argv)
     try:
         query(**vars(a))
